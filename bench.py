@@ -52,6 +52,8 @@ def parse_args():
     ap.add_argument("--verify-checksum", action="store_true", help="include the XXH64 kernel in the timed region")
     ap.add_argument("--no-other-configs", action="store_true", help="skip the config3/4/5 and config5_sharded keys")
     ap.add_argument("--no-link-ceiling", action="store_true", help="skip the raw H2D+D2H ceiling of the e2e record")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last step returned (a fixed, seeded "
+                    "sample of the frames: decoded bytes and result fields; rank 0) as DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -115,12 +117,30 @@ def make_workload(distinct, seed=1234):
     return frames, origs
 
 
+DUMP_FRAMES = 128  # frames --dump-outputs keeps: their decoded bytes as float32 come to 128 x 64 KiB x 4 B = 32 MiB
+
+
+def dump_pick(n):
+    """The frames --dump-outputs writes: a sample that depends on the batch size only, so two builds dump the same frames."""
+    return np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_FRAMES), replace=False))
+
+
+def dump_outputs(out_dir, pick, decoded, results):
+    """Write the sampled frames' outputs: frame_index.npy (which frames of the batch), decoded.npy (one row of decoded bytes per
+    frame, float32) and result_<field>.npy (each field of the frames' results, float64; RES_DT names the fields)."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "frame_index.npy"), pick.astype(np.float64))
+    np.save(os.path.join(out_dir, "decoded.npy"), decoded.astype(np.float32))
+    for name in results.dtype.names:
+        np.save(os.path.join(out_dir, f"result_{name}.npy"), results[name].astype(np.float64))
+
+
 # --------------------------------------------------------------------------------------------
 # reference arm: the oracle port on the host cores
 # --------------------------------------------------------------------------------------------
 def cpu_oracle_throughput(frames, origs, sample_frames, threads):
     """Decode `sample_frames` frames (the distinct set cycled) with the oracle on `threads` threads.
-    Returns (GB/s of decompressed bytes, seconds)."""
+    Returns (GB/s of decompressed bytes, seconds, decoded bytes, per-frame results)."""
     import oracle_lib as O
     L = O.lib()
     n = sample_frames
@@ -139,7 +159,7 @@ def cpu_oracle_throughput(frames, origs, sample_frames, threads):
     assert fails == 0
     k = n - 1
     assert out[k * FRAME_SIZE:(k + 1) * FRAME_SIZE].tobytes() == origs[k % d]
-    return n * FRAME_SIZE / dt / 1e9, dt
+    return n * FRAME_SIZE / dt / 1e9, dt, out, results
 
 
 def run_reference(args, rank, world):
@@ -152,8 +172,11 @@ def run_reference(args, rank, world):
         cpu_oracle_throughput(frames, origs, min(sample, 2048), threads)
     vals, times = [], []
     for _ in range(args.steps):
-        v, dt = cpu_oracle_throughput(frames, origs, sample, threads)
+        v, dt, out, results = cpu_oracle_throughput(frames, origs, sample, threads)
         vals.append(v); times.append(dt)
+    if args.dump_outputs:
+        pick = dump_pick(sample)
+        dump_outputs(args.dump_outputs, pick, out.reshape(sample, FRAME_SIZE)[pick], np.frombuffer(results, dtype=RES_DT)[pick])
     total_t = sum(times)
     value = args.steps * sample * FRAME_SIZE / total_t / 1e9
     desc = f"{sample} frames x 64 KiB per step ({len(frames)} distinct, cycled), oracle C port, {threads} threads"
@@ -255,6 +278,10 @@ def run_b200(args, rank, world, local_rank):
     res_np = results.cpu().numpy().view(np.dtype([("status", "<i4"), ("blocks", "<u4"), ("bytes_read", "<u8"), ("bytes_written", "<u8"),
                                                   ("content_size", "<u8"), ("window", "<u8"), ("chk_data", "<u4"), ("chk_calc", "<u4"),
                                                   ("has_chk", "<i4"), ("finished", "<i4")]))
+    if args.dump_outputs and rank == 0:
+        pick = dump_pick(n)
+        decoded = dst_all.view(n, FRAME_SIZE)[torch.from_numpy(pick).to(dev)].cpu().numpy()
+        dump_outputs(args.dump_outputs, pick, decoded, res_np[pick])
     assert (res_np["status"] == 0).all(), f"{int((res_np['status'] != 0).sum())} frames failed"
     assert (res_np["bytes_written"] == FRAME_SIZE).all() and (res_np["finished"] == 1).all()
     for k in list(range(0, min(n, d))) + [n - 1, n // 2]:
@@ -343,7 +370,7 @@ def run_b200(args, rank, world, local_rank):
     cpu = None
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         threads = os.cpu_count() or 1
-        v, dt = cpu_oracle_throughput(frames[:512], origs[:512], args.cpu_sample_frames, threads)
+        v, dt, _, _ = cpu_oracle_throughput(frames[:512], origs[:512], args.cpu_sample_frames, threads)
         cpu = {"value": v, "unit": "GB/s", "cores": threads, "kind": "port",
                "sample": f"{args.cpu_sample_frames} of the same frames ({dt:.1f} s wall), oracle C port, one frame per task"}
 
