@@ -14,9 +14,6 @@ constexpr int EXEC_WARPS = 4;
 #define EXEC_CTAS_PER_SM 7
 #endif
 constexpr uint32_t EXEC_ROW = 128;
-#ifndef EXEC_TILE_PATH
-#define EXEC_TILE_PATH 1
-#endif
 constexpr uint32_t EXEC_TILE = 1024;
 
 struct ExecWarpSmem {
@@ -25,9 +22,7 @@ struct ExecWarpSmem {
                              // [64] is the "past the end" pseudo segment
     unsigned long long segbase[66];  // indexed by id = segment index + 1: address of the source byte for output position 0
     uint32_t segthr[66];     // indexed by id: a byte at row-relative... see gather: fast iff (p - rlo) < segthr[id]
-#if EXEC_TILE_PATH
     __align__(16) uint8_t tile[EXEC_TILE + 48];  // a chunk's whole output span (sequence-centric path)
-#endif
     __align__(4) uint8_t rowmap[EXEC_ROW];  // (segment id + 1) at each non-empty segment's start byte inside the row
     __align__(4) uint8_t krow[EXEC_ROW];    // (segment id + 1) owning each row byte
 };
@@ -77,34 +72,18 @@ __device__ __forceinline__ void warp_fill(uint8_t* dst, uint8_t byte, uint32_t n
 
 // 16 source bytes starting at src (any alignment, GLOBAL memory) as four little-endian words.  Only the
 // aligned 32-bit words that hold one of the first n bytes are read.
-// As plain C ptxas turns the "needed?" chain into branches around the loads, which skip a word altogether when no lane needs it
-// (literal runs average three bytes: words 2..4 are almost never read).  -DCZB_EXEC_ASM_LD=1 makes every word one compare and one
-// predicated ld.global instead (no BSSY / BRA / BSYNC): measured SLOWER (k_exec 43.2 -> 44.4 ms per three waves), five always-issued
-// loads cost more than the branches.
+// The loads stay plain C: ptxas turns the "needed?" chain into branches that skip a word altogether when no lane needs it
+// (literal runs average three bytes: words 2..4 are almost never read), which measured faster than one predicated ld.global
+// per word (k_exec 43.2 against 44.4 ms per three waves).
 struct Vec16 { uint32_t v[4]; };
-#ifndef CZB_EXEC_ASM_LD
-#define CZB_EXEC_ASM_LD 0
-#endif
-template <bool CG, int K, int THR>  // word K of the vector's aligned source words, read iff x > THR
-__device__ __forceinline__ uint32_t ldg32_if_gt(const uint32_t* w, uint32_t x) {
-    uint32_t v;
-    if (CG) asm volatile("{\n\t.reg .pred p;\n\tsetp.gt.u32 p, %2, %4;\n\tmov.u32 %0, 0;\n\t@p ld.global.cg.u32 %0, [%1+%3];\n\t}" : "=r"(v) : "l"(w), "r"(x), "n"(4 * K), "n"(THR) : "memory");
-    else asm volatile("{\n\t.reg .pred p;\n\tsetp.gt.u32 p, %2, %4;\n\tmov.u32 %0, 0;\n\t@p ld.global.ca.u32 %0, [%1+%3];\n\t}" : "=r"(v) : "l"(w), "r"(x), "n"(4 * K), "n"(THR) : "memory");
-    return v;
-}
 template <bool CG = false>  // CG: read through L2 (data another warp of the CTA has just written)
 __device__ __forceinline__ Vec16 load16_unaligned(const uint8_t* __restrict__ src, uint32_t n) {
     const uintptr_t a = reinterpret_cast<uintptr_t>(src);
     const uint32_t mis = (uint32_t)(a & 3), sh = mis * 8, need = n + mis;
     const uint32_t* w = reinterpret_cast<const uint32_t*>(a & ~uintptr_t(3));
-#if CZB_EXEC_ASM_LD
-    const uint32_t w0 = ldg32_if_gt<CG, 0, 0>(w, n);
-    const uint32_t w1 = ldg32_if_gt<CG, 1, 4>(w, need), w2 = ldg32_if_gt<CG, 2, 8>(w, need), w3 = ldg32_if_gt<CG, 3, 12>(w, need), w4 = ldg32_if_gt<CG, 4, 16>(w, need);
-#else
     auto ld = [&](int k) -> uint32_t { return CG ? __ldcg(w + k) : w[k]; };
     const uint32_t w0 = n ? ld(0) : 0u;
     const uint32_t w1 = need > 4 ? ld(1) : 0u, w2 = need > 8 ? ld(2) : 0u, w3 = need > 12 ? ld(3) : 0u, w4 = need > 16 ? ld(4) : 0u;
-#endif
     Vec16 r;
     r.v[0] = __funnelshift_r(w0, w1, sh); r.v[1] = __funnelshift_r(w1, w2, sh);
     r.v[2] = __funnelshift_r(w2, w3, sh); r.v[3] = __funnelshift_r(w3, w4, sh);
@@ -117,9 +96,6 @@ __device__ __forceinline__ Vec16 load16_unaligned(const uint8_t* __restrict__ sr
 // 72-register cap): 4 instructions per byte instead of 3 on the integer pipe that issues one instruction per two cycles.
 // No "memory" clobber on the stores (the loads of the next vector may move across them); tile_stores_done() orders them
 // before anything that reads the tile.
-#ifndef CZB_EXEC_ASM_ST
-#define CZB_EXEC_ASM_ST 1
-#endif
 __device__ __forceinline__ uint32_t tile_addr(const uint8_t* t) {
     uint32_t a = (uint32_t)__cvta_generic_to_shared(t);
     asm volatile("" : "+r"(a));  // opaque: one register, not a sum to re-form
@@ -136,21 +112,11 @@ __device__ __forceinline__ void store4_to_tile(uint32_t a, uint32_t w, uint32_t 
     sts_u8_if<4 * G>(a, w, n); sts_u8_if<4 * G + 1>(a, w >> 8, n); sts_u8_if<4 * G + 2>(a, w >> 16, n); sts_u8_if<4 * G + 3>(a, w >> 24, n);
 }
 __device__ __forceinline__ void store16_to_tile(uint8_t* t, const Vec16& x, uint32_t n) {
-#if CZB_EXEC_ASM_ST
     const uint32_t a = tile_addr(t);
     store4_to_tile<0>(a, x.v[0], n);
     if (__any_sync(0xFFFFFFFFu, n > 4u)) store4_to_tile<1>(a, x.v[1], n);
     if (__any_sync(0xFFFFFFFFu, n > 8u)) store4_to_tile<2>(a, x.v[2], n);
     if (__any_sync(0xFFFFFFFFu, n > 12u)) store4_to_tile<3>(a, x.v[3], n);
-#else
-#pragma unroll
-    for (int g = 0; g < 4; g++) {
-        if (g == 0 || __any_sync(0xFFFFFFFFu, n > 4u * g)) {
-#pragma unroll
-            for (int k = 4 * g; k < 4 * g + 4; k++) if ((uint32_t)k < n) t[k] = (uint8_t)(x.v[g] >> (8 * (k & 3)));
-        }
-    }
-#endif
 }
 
 // All lanes copy n bytes src -> tile + dst_off for the lane `j` that owns the job (arguments are taken from lane j).
@@ -164,23 +130,47 @@ __device__ __forceinline__ void coop_copy_to_tile(uint8_t* tile, unsigned lane, 
 
 // the same without the votes
 __device__ __forceinline__ void store16_to_tile_all(uint8_t* t, const Vec16& x, uint32_t n) {
-#if CZB_EXEC_ASM_ST
     const uint32_t a = tile_addr(t);
     store4_to_tile<0>(a, x.v[0], n); store4_to_tile<1>(a, x.v[1], n); store4_to_tile<2>(a, x.v[2], n); store4_to_tile<3>(a, x.v[3], n);
-#else
-#pragma unroll
-    for (int k = 0; k < 16; k++) if ((uint32_t)k < n) t[k] = (uint8_t)(x.v[k >> 2] >> (8 * (k & 3)));
-#endif
 }
 
-// Sequence-centric execution of one chunk whose output span fits the tile: lane = sequence.  The first 16 bytes of
-// every literal run and of every match whose source is already in dst are copied by their own lane (all lanes in
-// parallel, uniform control flow); tails and the matches that depend on output not yet in dst are done by the whole
-// warp, one at a time, in sequence order.  The tile is flushed with aligned 16-byte stores.
-//
-// avail_rel (<= 0) and wait_prev exist for k_exec_big, where several warps work on consecutive chunks of one frame:
-// output below obase + avail_rel is complete in dst when the call starts; wait_prev() returns once everything
-// below obase is.  The one-warp-per-frame kernel passes 0 and a no-op.
+// Wrapping windows (k_exec_big, k_exec_flow): WIN bytes of shared memory (a power of two, 16-byte aligned) that hold
+// position p at win[p % WIN].  The first n (<= 16) bytes from position p: aligned words and funnel shifts, word indices wrapped.
+template <uint32_t WIN>
+__device__ __forceinline__ Vec16 win_load16(const uint8_t* win, uint32_t p, uint32_t n) {
+    const uint32_t mis = p & 3u, sh = mis * 8u, need = n + mis;
+    const uint32_t* w32 = reinterpret_cast<const uint32_t*>(win);
+    const uint32_t wi = p >> 2;
+    auto ld = [&](uint32_t k) -> uint32_t { return w32[(wi + k) & (WIN / 4 - 1)]; };
+    const uint32_t w0 = n ? ld(0) : 0u;
+    const uint32_t w1 = need > 4 ? ld(1) : 0u, w2 = need > 8 ? ld(2) : 0u, w3 = need > 12 ? ld(3) : 0u, w4 = need > 16 ? ld(4) : 0u;
+    Vec16 r;
+    r.v[0] = __funnelshift_r(w0, w1, sh); r.v[1] = __funnelshift_r(w1, w2, sh);
+    r.v[2] = __funnelshift_r(w2, w3, sh); r.v[3] = __funnelshift_r(w3, w4, sh);
+    return r;
+}
+// Positions [p, p + n) = the first n (<= 16) bytes of v.  When no lane's sixteen bytes wrap around the window's end (all but one
+// vector in WIN / 16): one address per lane and immediate offsets, as in store16_to_tile; otherwise byte stores at wrapped indices.
+template <uint32_t WIN>
+__device__ __forceinline__ void win_store16(uint8_t* win, uint32_t p, const Vec16& v, uint32_t n) {
+    if (__all_sync(0xFFFFFFFFu, (p & (WIN - 1)) <= WIN - 16u)) {
+        const uint32_t a = tile_addr(win) + (p & (WIN - 1));
+        store4_to_tile<0>(a, v.v[0], n);
+        if (__any_sync(0xFFFFFFFFu, n > 4u)) store4_to_tile<1>(a, v.v[1], n);
+        if (__any_sync(0xFFFFFFFFu, n > 8u)) store4_to_tile<2>(a, v.v[2], n);
+        if (__any_sync(0xFFFFFFFFu, n > 12u)) store4_to_tile<3>(a, v.v[3], n);
+        tile_stores_done();
+        return;
+    }
+#pragma unroll
+    for (int g = 0; g < 4; g++) {
+        if (g == 0 || __any_sync(0xFFFFFFFFu, n > 4u * g)) {
+#pragma unroll
+            for (int k = 4 * g; k < 4 * g + 4; k++) if ((uint32_t)k < n) win[(p + k) & (WIN - 1)] = (uint8_t)(v.v[g] >> (8 * (k & 3)));
+        }
+    }
+}
+
 // Which frames get a whole CTA (k_exec_big) instead of one warp (k_exec):
 //  * large ones (>= 2^big_cls compressed bytes) with sparse sequences (>= big_seq_bytes compressed bytes per sequence:
 //    literal-heavy data, long matches), whose warps rarely wait for each other (1 MiB literal-heavy frames 253 -> 400 GB/s);
@@ -193,7 +183,6 @@ __device__ __forceinline__ bool frame_is_big(const FrameInfo& fi, const BigRule&
     return (fi.size_cls >= r.big_cls && fi.n_seq * r.big_seq_bytes <= fi.src_end) || (fi.size_cls >= r.share_cls && fi.src_end >= r.share_bytes);
 }
 
-struct NoWait { __device__ __forceinline__ void operator()() const {} };
 // Measurement aid (-DCZB_BIG_CLOCK): cycles per phase of k_exec_big, accumulated by thread 0 of CTA 0 and printed per launch.
 #ifdef CZB_BIG_CLOCK
 __device__ unsigned long long czb_dbg_clk[16];
@@ -201,14 +190,19 @@ __device__ unsigned long long czb_dbg_clk[16];
 #else
 #define CLK_MARK(k) do { } while (0)
 #endif
-template <bool CG_LOADS, typename WaitPrev>
+// Sequence-centric execution of one chunk whose output span fits the tile: lane = sequence.  Everything below obase is
+// complete in dst when the call starts.  The first 16 bytes of every literal run and of every match whose source is
+// already in dst are copied by their own lane (all lanes in parallel, uniform control flow); tails and the matches that
+// read this chunk's own output are done by the whole warp, one at a time, in sequence order.  The tile is flushed with
+// aligned 16-byte stores.  CG_LOADS: match sources are read through L2 (another warp of the CTA may have just written them).
+template <bool CG_LOADS>
 __device__ __forceinline__ void exec_chunk_tile(uint8_t* tile_base, uint8_t* obase, const uint8_t* __restrict__ lits, bool lit_rle,
                                                 uint32_t rle_byte, unsigned lane, uint32_t ll, uint32_t ml, uint32_t off,
-                                                uint32_t my_lit, uint32_t segA, uint32_t span, int avail_rel, WaitPrev wait_prev) {
+                                                uint32_t my_lit, uint32_t segA, uint32_t span) {
     const uint32_t a0 = (uint32_t)(reinterpret_cast<uintptr_t>(obase) & 15);
     uint8_t* tile = tile_base + a0;  // tile[p] = output byte at chunk-relative position p
     const uint32_t segM = segA + ll;
-    const bool indep = ml > 0 && (int)(segM + ml) - (int)off <= avail_rel;  // whole source is already in dst
+    const bool indep = ml > 0 && (int)(segM + ml) - (int)off <= 0;  // the whole source ends at or below the chunk start: already in dst
     const uint8_t* msrc = obase + ((int64_t)segM - (int64_t)off);
     // first 16 bytes of every literal run and independent match: all loads are issued before the stores
     {
@@ -226,11 +220,10 @@ __device__ __forceinline__ void exec_chunk_tile(uint8_t* tile_base, uint8_t* oba
     for (unsigned m = __ballot_sync(0xFFFFFFFFu, indep && ml > 16u); m; m &= m - 1)
         coop_copy_to_tile<CG_LOADS>(tile, lane, __ffs(m) - 1, segM + 16u, msrc + 16, ml - 16u);
     __syncwarp();
-    wait_prev();
     bool done = indep || ml == 0;
     if (CG_LOADS) {
-        // k_exec_big: everything below obase is in dst now.  Matches whose source ends there but was not available
-        // when the chunk started are mutually independent: one more per-lane pass instead of one warp pass each.
+        // A match whose source ends below obase but which the signed test above did not take (an offset of 2^31 or more,
+        // which the callers' checks rule out) is copied from dst in one more per-lane pass.
         const bool late = !done && segM + ml <= off;
         const uint32_t nm = late ? (ml < 16u ? ml : 16u) : 0u;
         if (__any_sync(0xFFFFFFFFu, late)) {

@@ -21,17 +21,12 @@
 // HBM traffic per frame: literals + 8 B/sequence in, decoded bytes out; match sources are recent output (L1/L2 when the
 // in-flight working set allows, DRAM otherwise: profiles/r01_final_ncu_summary.md).
 #include <cstdio>
-#include <cstdlib>
 
 #include "czb_exec.cuh"
 #include "czb_internal.cuh"
 
 namespace czb {
 
-#ifndef CZB_EXEC_PF
-#define CZB_EXEC_PF 0
-#endif
-#if EXEC_TILE_PATH
 // ---- k_exec_big's chunk executor: the frame's recent output lives in a shared-memory window ----
 // k_exec_big commits the chunks of a frame in order, so whatever a chunk does between "everything before me is
 // complete" and "I am complete" is a serial chain that every other warp of the CTA waits for.  With the chunk built in
@@ -65,43 +60,13 @@ struct WinView {
     __device__ __forceinline__ uint32_t idx(int x) const { return (gb + (uint32_t)x) & BIG_WIN_MASK; }
     __device__ __forceinline__ uint8_t rd(int x) const { return x >= lo_rel ? win[idx(x)] : __ldcg(obase + x); }
     // first n (<= 16) bytes from position x, which lie in the window
-    __device__ __forceinline__ Vec16 load16(int x, uint32_t n) const {
-        const uint32_t a = gb + (uint32_t)x, mis = a & 3u, sh = mis * 8u, need = n + mis;
-        const uint32_t* w32 = reinterpret_cast<const uint32_t*>(win);
-        const uint32_t wi = a >> 2;
-        auto ld = [&](uint32_t k) -> uint32_t { return w32[(wi + k) & (BIG_WIN / 4 - 1)]; };
-        const uint32_t w0 = n ? ld(0) : 0u;
-        const uint32_t w1 = need > 4 ? ld(1) : 0u, w2 = need > 8 ? ld(2) : 0u, w3 = need > 12 ? ld(3) : 0u, w4 = need > 16 ? ld(4) : 0u;
-        Vec16 r;
-        r.v[0] = __funnelshift_r(w0, w1, sh); r.v[1] = __funnelshift_r(w1, w2, sh);
-        r.v[2] = __funnelshift_r(w2, w3, sh); r.v[3] = __funnelshift_r(w3, w4, sh);
-        return r;
-    }
-    __device__ __forceinline__ void store16(int x, const Vec16& v, uint32_t n) const {
-        const uint32_t a = gb + (uint32_t)x;
-#if CZB_EXEC_ASM_ST
-        // no lane's sixteen bytes wrap around the window's end: one address per lane and immediate offsets (see store16_to_tile)
-        if (__all_sync(0xFFFFFFFFu, (a & BIG_WIN_MASK) <= BIG_WIN - 16u)) {
-            const uint32_t sa = tile_addr(win) + (a & BIG_WIN_MASK);
-            store4_to_tile<0>(sa, v.v[0], n);
-            if (__any_sync(0xFFFFFFFFu, n > 4u)) store4_to_tile<1>(sa, v.v[1], n);
-            if (__any_sync(0xFFFFFFFFu, n > 8u)) store4_to_tile<2>(sa, v.v[2], n);
-            if (__any_sync(0xFFFFFFFFu, n > 12u)) store4_to_tile<3>(sa, v.v[3], n);
-            tile_stores_done();
-            return;
-        }
-#endif
-#pragma unroll
-        for (int g = 0; g < 4; g++) {
-            if (g == 0 || __any_sync(0xFFFFFFFFu, n > 4u * g)) {
-#pragma unroll
-                for (int k = 4 * g; k < 4 * g + 4; k++) if ((uint32_t)k < n) win[(a + k) & BIG_WIN_MASK] = (uint8_t)(v.v[g] >> (8 * (k & 3)));
-            }
-        }
-    }
+    __device__ __forceinline__ Vec16 load16(int x, uint32_t n) const { return win_load16<BIG_WIN>(win, gb + (uint32_t)x, n); }
+    __device__ __forceinline__ void store16(int x, const Vec16& v, uint32_t n) const { win_store16<BIG_WIN>(win, gb + (uint32_t)x, v, n); }
 };
 
-// Same contract as exec_chunk_tile (lane = sequence, chunk span <= EXEC_TILE); publish() commits the chunk.
+// Same contract as exec_chunk_tile (lane = sequence, chunk span <= EXEC_TILE), except that only output below obase + avail_rel
+// (avail_rel <= 0) is complete in dst when the call starts; wait_prev() returns once everything below obase is, and publish()
+// commits the chunk.
 template <typename WaitPrev, typename Publish>
 __device__ __forceinline__ void exec_chunk_win(uint8_t* win, uint8_t* obase, int lo_rel, const uint8_t* __restrict__ lits, bool lit_rle,
                                                uint32_t rle_byte, unsigned lane, uint32_t ll, uint32_t ml, uint32_t off,
@@ -181,7 +146,6 @@ __device__ __forceinline__ void exec_chunk_win(uint8_t* win, uint8_t* obase, int
     __syncwarp();
     CLK_MARK(6);
 }
-#endif
 
 __global__ void __launch_bounds__(EXEC_WARPS * 32, EXEC_MIN_CTAS) k_exec(const czb_frame_desc* __restrict__ descs, const FrameInfo* __restrict__ infos,
                                                            BigRule rule, uint32_t n_exec, WaveCounters* __restrict__ counters, const uint32_t* __restrict__ exec_order,
@@ -245,19 +209,11 @@ __global__ void __launch_bounds__(EXEC_WARPS * 32, EXEC_MIN_CTAS) k_exec(const c
             const Seq* seqs = seq_scratch + d.seq_off;
             // records are read exactly once: stream them (evict-first) so that L2 keeps the frame's recent output instead
             Seq rec_next = lane < d.n_seq ? __ldcs(seqs + lane) : 0ull;
-#if CZB_EXEC_PF
-            Seq rec_next2 = lane + 32 < d.n_seq ? __ldcs(seqs + lane + 32) : 0ull;  // two chunks ahead: the next chunk's record is in registers when this one runs
-#endif
             for (uint32_t s0 = 0; s0 < d.n_seq; s0 += 32) {
                 const uint32_t i = s0 + lane;
                 const bool have = i < d.n_seq;
                 const Seq rec = rec_next;
-#if CZB_EXEC_PF
-                rec_next = rec_next2;
-                rec_next2 = i + 64 < d.n_seq ? __ldcs(seqs + i + 64) : 0ull;
-#else
                 if (i + 32 < d.n_seq) rec_next = __ldcs(seqs + i + 32);  // next chunk's record is in flight while this chunk executes
-#endif
                 uint32_t ll = 0, ml = 0, off = 1;
                 if (have) { ll = seq_ll(rec); ml = seq_ml(rec); off = off29_resolve(seq_off29(rec), h0, h1, h2); }
                 // warp prefix sums: literal offsets and output offsets (u32 cannot wrap: 32 * (131071 + 131074) < 2^32)
@@ -289,27 +245,11 @@ __global__ void __launch_bounds__(EXEC_WARPS * 32, EXEC_MIN_CTAS) k_exec(const c
                     const unsigned errm = __ballot_sync(0xFFFFFFFFu, err != CZS_OK);
                     if (errm) { status = __shfl_sync(0xFFFFFFFFu, err, __ffs(errm) - 1); break; }
                 }
-#if CZB_EXEC_PF
-                {   // L2 prefetch of the NEXT chunk's match sources that lie below this chunk (already in dst, possibly evicted to DRAM:
-                    // 4144 frames x 64 KiB in flight exceed the L2): no destination register, the line is in L2 when the next chunk loads it
-                    const bool have2 = i + 32 < d.n_seq;
-                    const uint32_t ll2 = have2 ? seq_ll(rec_next) : 0u, ml2 = have2 ? seq_ml(rec_next) : 0u;
-                    const uint32_t off2 = have2 ? off29_resolve(seq_off29(rec_next), h0, h1, h2) : 1u;
-                    uint32_t o2 = ll2 + ml2;
-#pragma unroll
-                    for (int o = 1; o < 32; o <<= 1) { const uint32_t a = __shfl_up_sync(0xFFFFFFFFu, o2, o); if ((int)lane >= o) o2 += a; }
-                    const uint32_t segM2 = span + o2 - ml2;  // relative to this chunk's base
-                    if (ml2 && off2 > segM2 && (uint64_t)off2 <= out + segM2)
-                        asm volatile("prefetch.global.L2 [%0];" ::"l"(dst + out + segM2 - off2));
-                }
-#endif
-#if EXEC_TILE_PATH
                 if (span <= EXEC_TILE) {  // the common case: short segments, span of a few hundred bytes
-                    exec_chunk_tile<false>(sm.tile, dst + out, lits, lit_rle, rle_byte, lane, ll, ml, off, my_lit, my_out, span, 0, NoWait{});
+                    exec_chunk_tile<false>(sm.tile, dst + out, lits, lit_rle, rle_byte, lane, ll, ml, off, my_lit, my_out, span);
                     out += span; lit_pos += lit_used;
                     continue;
                 }
-#endif
                 // general path (long segments): publish the 64 segments of this chunk
                 const uint32_t segA = my_out, segM = my_out + ll;
                 sm.bound[2 * lane] = segA; sm.bound[2 * lane + 1] = segM;
@@ -456,10 +396,6 @@ __global__ void __launch_bounds__(EXEC_WARPS * 32, EXEC_MIN_CTAS) k_exec(const c
 //     committed and are then done in sequence order by the whole warp, exactly as in k_exec.
 // Same checks, same statuses, same results as k_exec; the first failing chunk in sequence order wins.
 // ---------------------------------------------------------------------------------------
-#ifndef CZB_BIG_WIN
-#define CZB_BIG_WIN 1  // 0: always the tile + dst hand-over (measurement aid)
-#endif
-constexpr bool BIG_USE_WIN = CZB_BIG_WIN != 0;
 #ifndef CZB_BIG_POLL_NS
 #define CZB_BIG_POLL_NS 32
 #endif
@@ -472,13 +408,13 @@ constexpr int BIG_WARPS = CZB_BIG_WARPS;
 #define CZB_BIG_MIN_CTAS 7  // 72 registers, no spills; ~25 KB of shared memory per CTA
 #endif
 constexpr int BIG_MIN_CTAS = CZB_BIG_MIN_CTAS;
-static_assert(BIG_WARPS <= BIG_WARPS_MAX && BIG_WARPS * (EXEC_TILE + 48) <= BIG_WIN, "window reach and tile carve-out assume at most BIG_WARPS_MAX warps");
+static_assert(BIG_WARPS <= BIG_WARPS_MAX, "the window reach assumes at most BIG_WARPS_MAX warps");
 constexpr uint32_t BIG_BATCH = 1024;  // chunks per batch (n_seq <= 0x7F00 + 0xFFFF, sequence_section.cairo: at most 3065 chunks per block)
 
 struct BigSmem {
     uint32_t chunk_lit[BIG_BATCH + 4];  // exclusive prefix of literal bytes per chunk of the batch, [n] = batch total
     uint32_t chunk_out[BIG_BATCH + 4];  // exclusive prefix of output bytes per chunk of the batch
-    __align__(16) uint8_t win[BIG_WIN];      // recent output of the current block (exec_chunk_win); per-warp tiles for a block with long chunks
+    __align__(16) uint8_t win[BIG_WIN];      // recent output of the current block (exec_chunk_win); warp 0's tile for a chunk longer than a slice
     unsigned long long committed_out;        // every output byte below this offset is complete (in the window or in dst)
     uint32_t n_long;                         // chunks of the current batch that are longer than a window slice
     uint16_t long_idx[BIG_BATCH];            // their indices, ascending
@@ -489,11 +425,7 @@ struct BigSmem {
 
 // __threadfence_block() is membar.cta = fence.sc.cta, a sequentially consistent fence: several hundred cycles each, and
 // k_exec_big has four of them on every chunk.  Acquire/release ordering is all the commit protocol needs.
-#ifndef CZB_BIG_SC_FENCE
 __device__ __forceinline__ void fence_cta() { asm volatile("fence.acq_rel.cta;" ::: "memory"); }
-#else
-__device__ __forceinline__ void fence_cta() { __threadfence_block(); }
-#endif
 
 __device__ __forceinline__ void cta_copy(uint8_t* dst, const uint8_t* src, uint64_t n, unsigned warp) {
     const uint64_t per = ((n + BIG_WARPS - 1) / BIG_WARPS + 15) & ~15ull;
@@ -679,16 +611,9 @@ __global__ void __launch_bounds__(BIG_WARPS * 32, BIG_MIN_CTAS) k_exec_big(const
                     fence_cta();
                     const uint64_t behind = out_c - (avail < out_c ? avail : out_c);
                     const int avail_rel = -(int)(behind < 0x40000000ull ? behind : 0x40000000ull);
-                    if (BIG_USE_WIN) {
-                        const uint32_t in_run = sm.chunk_out[q] - seg_out0;  // bytes of this run before the chunk: all of them went through the window
-                        const int lo_rel = -(int)(in_run < (uint32_t)BIG_WIN_REACH ? in_run : (uint32_t)BIG_WIN_REACH);
-                        exec_chunk_win(sm.win, dst + out_c, lo_rel, lits, lit_rle, rle_byte, lane, ll, ml, off, my_lit, my_out, span, avail_rel, wait_prev, publish, dbg);
-                    } else {
-                        exec_chunk_tile<true>(sm.win + warp * (EXEC_TILE + 48), dst + out_c, lits, lit_rle, rle_byte, lane, ll, ml, off, my_lit, my_out, span, avail_rel, wait_prev);
-                        __syncwarp();
-                        fence_cta();  // the flushed bytes are visible to the CTA before the commit
-                        publish();
-                    }
+                    const uint32_t in_run = sm.chunk_out[q] - seg_out0;  // bytes of this run before the chunk: all of them went through the window
+                    const int lo_rel = -(int)(in_run < (uint32_t)BIG_WIN_REACH ? in_run : (uint32_t)BIG_WIN_REACH);
+                    exec_chunk_win(sm.win, dst + out_c, lo_rel, lits, lit_rle, rle_byte, lane, ll, ml, off, my_lit, my_out, span, avail_rel, wait_prev, publish, dbg);
                 } else {
                     // A chunk that does not fit a slice: once everything before it is in dst, it is cut at sequence boundaries
                     // into pieces that do fit (each executed like a chunk of its own, through a tile, with the lanes outside
@@ -717,7 +642,7 @@ __global__ void __launch_bounds__(BIG_WARPS * 32, BIG_MIN_CTAS) k_exec_big(const
                             const bool in = lane >= start && lane <= last;
                             const uint32_t span_p = __shfl_sync(0xFFFFFFFFu, my_out + ll + ml, last) - base_o;
                             exec_chunk_tile<true>(sm.win, dst + out_c + base_o, lits, lit_rle, rle_byte, lane, in ? ll : 0u, in ? ml : 0u, off, my_lit,
-                                                  in ? my_out - base_o : 0u, span_p, 0, NoWait{});
+                                                  in ? my_out - base_o : 0u, span_p);
                             start = last + 1;
                         }
                         __syncwarp();
@@ -822,7 +747,6 @@ void launch_exec(const LaunchCtx& lc, const ExecSide& side, int sm_count, const 
 }
 
 int setup_exec_attributes() {
-    if (const char* e = getenv("CZB_EXEC_CARVEOUT")) cudaFuncSetAttribute(k_exec, cudaFuncAttributePreferredSharedMemoryCarveout, atoi(e));  // tuning knob (percent)
     return (int)cudaFuncSetAttribute(k_exec_big, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(BigSmem));
 }
 

@@ -126,41 +126,8 @@ struct FlowWin {
     uint8_t* win;
     __device__ __forceinline__ uint8_t rd(uint32_t p) const { return win[p & FLOW_WIN_MASK]; }
     __device__ __forceinline__ void wr(uint32_t p, uint8_t v) const { win[p & FLOW_WIN_MASK] = v; }
-    // first n (<= 16) bytes from position p
-    __device__ __forceinline__ Vec16 load16(uint32_t p, uint32_t n) const {
-        const uint32_t mis = p & 3u, sh = mis * 8u, need = n + mis;
-        const uint32_t* w32 = reinterpret_cast<const uint32_t*>(win);
-        const uint32_t wi = p >> 2;
-        auto ld = [&](uint32_t k) -> uint32_t { return w32[(wi + k) & (FLOW_WIN / 4 - 1)]; };
-        const uint32_t w0 = n ? ld(0) : 0u;
-        const uint32_t w1 = need > 4 ? ld(1) : 0u, w2 = need > 8 ? ld(2) : 0u, w3 = need > 12 ? ld(3) : 0u, w4 = need > 16 ? ld(4) : 0u;
-        Vec16 r;
-        r.v[0] = __funnelshift_r(w0, w1, sh); r.v[1] = __funnelshift_r(w1, w2, sh);
-        r.v[2] = __funnelshift_r(w2, w3, sh); r.v[3] = __funnelshift_r(w3, w4, sh);
-        return r;
-    }
-    __device__ __forceinline__ void store16(uint32_t p, const Vec16& v, uint32_t n) const {
-#if CZB_EXEC_ASM_ST
-        // No lane's sixteen bytes wrap around the window's end (all but one vector in FLOW_WIN / 16): one address per lane, immediate offsets,
-        // the byte predicates inside the asm (czb_exec.cuh) instead of an add, a mask and an add per byte.
-        if (__all_sync(0xFFFFFFFFu, (p & FLOW_WIN_MASK) <= FLOW_WIN - 16u)) {
-            const uint32_t a = tile_addr(win) + (p & FLOW_WIN_MASK);
-            store4_to_tile<0>(a, v.v[0], n);
-            if (__any_sync(0xFFFFFFFFu, n > 4u)) store4_to_tile<1>(a, v.v[1], n);
-            if (__any_sync(0xFFFFFFFFu, n > 8u)) store4_to_tile<2>(a, v.v[2], n);
-            if (__any_sync(0xFFFFFFFFu, n > 12u)) store4_to_tile<3>(a, v.v[3], n);
-            tile_stores_done();
-            return;
-        }
-#endif
-#pragma unroll
-        for (int g = 0; g < 4; g++) {
-            if (g == 0 || __any_sync(0xFFFFFFFFu, n > 4u * g)) {
-#pragma unroll
-                for (int k = 4 * g; k < 4 * g + 4; k++) if ((uint32_t)k < n) win[(p + k) & FLOW_WIN_MASK] = (uint8_t)(v.v[g] >> (8 * (k & 3)));
-            }
-        }
-    }
+    __device__ __forceinline__ Vec16 load16(uint32_t p, uint32_t n) const { return win_load16<FLOW_WIN>(win, p, n); }
+    __device__ __forceinline__ void store16(uint32_t p, const Vec16& v, uint32_t n) const { win_store16<FLOW_WIN>(win, p, v, n); }
 };
 
 __global__ void __launch_bounds__(FLOW_WARPS * 32, FLOW_P_MIN_CTAS) k_exec_flow(const czb_frame_desc* __restrict__ descs, const FrameInfo* __restrict__ infos,
@@ -356,7 +323,7 @@ __global__ void __launch_bounds__(FLOW_WARPS * 32, FLOW_P_MIN_CTAS) k_exec_flow(
                                     const bool in = lane >= start && lane <= last;
                                     const uint32_t span_p = __shfl_sync(0xFFFFFFFFu, rel + ll + ml, last) - base_o;
                                     exec_chunk_tile<true>(sm.long_tile, obase + base_o, lits, lit_rle, rle_byte, lane, in ? ll : 0u, in ? ml : 0u, off, my_lit,
-                                                          in ? rel - base_o : 0u, span_p, 0, NoWait{});
+                                                          in ? rel - base_o : 0u, span_p);
                                     start = last + 1;
                                 }
                                 __syncwarp();

@@ -25,9 +25,6 @@ namespace czb {
 #define CZB_FSE_WARPS 4  // table-building warps per CTA (6 / 8 measured: see DESIGN.md)
 #endif
 constexpr int FSE_WARPS = CZB_FSE_WARPS;
-#ifndef CZB_FSE_QUAD
-#define CZB_FSE_QUAD 1  // four records leave as two 16-byte stores (half the store sectors); 0: one 8-byte store per sequence
-#endif
 #ifndef CZB_FSE_SLOTS
 #define CZB_FSE_SLOTS 27
 #endif
@@ -54,20 +51,11 @@ struct alignas(16) FseWarpTmp {
     int16_t probs[FSE_MAX_SYMBOLS];
     uint8_t rank_sym[1 << FSE_MAX_LOG];
 };
-static_assert(sizeof(FseWarpTmp) * FSE_WARPS >= FSE_SLOTS * (RevBitsWin::RING + 16 + 4) + 16, "phase-2 rings (+ a 16-byte mirror and one word per lane, one 16-byte dummy slot) reuse phase-1 scratch");
+static_assert(sizeof(FseWarpTmp) * FSE_WARPS >= FSE_SLOTS * (RevBitsWin::RING + 16) + 16, "phase-2 rings (+ a 16-byte mirror per lane, one 16-byte dummy slot) reuse phase-1 scratch");
 
-#ifndef CZB_FSE_SPLIT
-#define CZB_FSE_SPLIT 0  // 0: one warp, lean step (default); 1: the step split over two warps (state machine | values, history, records: measured no faster); 2: one warp, round-1 step
-#endif
-[[maybe_unused]] constexpr int FSE_HAND_STEPS = 4;  // steps per hand-over buffer: one barrier pair and three 16-byte vectors per lane
 struct FseSmem {
     uint16_t entries[FSE_SLOTS * FSE_SLOT_ENTRIES + 64 + 32 + 64];  // per-slot tables, then predefined LL, OF, ML
-    union {
-        FseSlot slot[FSE_SLOTS];
-        // split decode: two buffers of FSE_HAND_STEPS steps x {bits hi, bits lo, codes} per lane, laid out [buffer][vector][lane]
-        // (lane stride 16 bytes: conflict-free).  The slots are dead by then: both warps copied theirs into registers.
-        uint4 hand[2][3][FSE_SLOTS];
-    };
+    FseSlot slot[FSE_SLOTS];
     FseWarpTmp tmp[FSE_WARPS];
     uint32_t ll_code[64];  // base | bits << 27 (lookup_ll_code :299-345); bit 20 = code beyond the table -> (0,255)
     uint32_t ml_code[64];  // (lookup_ml_code :347-395)
@@ -79,7 +67,7 @@ __device__ __constant__ uint8_t kLLBits[36] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 
 __device__ __constant__ uint32_t kMLBase[53] = {3, 4, 5, 6, 7, 8, 9, 10, 11, 12, 13, 14, 15, 16, 17, 18, 19, 20, 21, 22, 23, 24, 25, 26, 27, 28, 29, 30, 31, 32, 33, 34, 35, 37, 39, 41, 43, 47, 51, 59, 67, 83, 99, 131, 259, 515, 1027, 2051, 4099, 8195, 16387, 32771, 65539};
 __device__ __constant__ uint8_t kMLBits[53] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 1, 1, 1, 1, 2, 2, 3, 3, 4, 4, 5, 7, 8, 9, 10, 11, 12, 13, 14, 15, 16};
 
-constexpr uint32_t FSE_BAD_CODE = 1u << 20;  // in ll_code / ml_code entries; an offset code >= 32 shifted left by 15 lands on the same bit
+constexpr uint32_t FSE_BAD_CODE = 1u << 20;  // in ll_code / ml_code entries: a code beyond the table
 __device__ __forceinline__ int stream_max_log(int s) { return s == 1 ? 8 : 9; }  // LL 9, OF 8, ML 9 (:397-399)
 
 // Bytes a table description of `mode` occupies at p (for skipping to a later stream's description).
@@ -214,257 +202,6 @@ __global__ void __launch_bounds__(FSE_WARPS * 32, 3) k_fse(const czb_frame_desc*
         }
     }
     __syncthreads();
-#if CZB_FSE_SPLIT == 1
-    if (warp >= 2) return;
-    // ---- phase 2, split over two warps; lane = block in both ----
-    // The decode step is one dependency chain per block, and the warp that walks it is alone on its scheduler: a step costs
-    // its instruction count (154 SASS instructions, ~250 cycles when one warp did everything).  Only the state machine is
-    // on that chain -- codes -> bit counts -> position -> next states.  Warp 0 ("walker") does just that and hands every
-    // step's 64 unread bits and three codes to warp 1 ("packer") through shared memory; the packer extracts the values,
-    // runs the offset history (do_offset_history), packs and stores the records, and owns the block's result.  Hand-over:
-    // two buffers of four steps, named barriers full/empty per buffer (bar.arrive / bar.sync producer-consumer pairs).
-    // Both warps keep all 32 lanes alive in the loop (barriers are warp-wide); a lane whose block cannot take the fast
-    // path (status, padding, missing table) or that hits trouble on it is decoded afterwards by the packer with the exact
-    // one-warp loop below, which reports the reference's first error.
-    const bool has = lane < FSE_SLOTS;
-    FseSlot slc = sm.slot[has ? lane : 0];
-    if (!has) { slc.blk = NONE32; slc.n_seq = 0; slc.status = CZS_NOT_DECODED; }
-    const FseSlot& sl = slc;
-    // phase 1's scratch is dead now: per lane a 128-byte bitstream ring with a 16-byte mirror of its top below it (the walker
-    // reads four consecutive words downwards from any ring word without wrapping its addresses), then one 16-byte slot that
-    // absorbs the refills that have nothing to fetch, then one word per lane for what the walker tells the packer
-    constexpr uint32_t RING_STRIDE = RevBitsWin::RING + 16;
-    uint32_t* misc = reinterpret_cast<uint32_t*>(reinterpret_cast<uint8_t*>(sm.tmp) + FSE_SLOTS * RING_STRIDE + 16);
-    const uint32_t ring_addr = (uint32_t)__cvta_generic_to_shared(sm.tmp) + lane * RING_STRIDE + 16u;
-    const uint32_t dummy = (uint32_t)__cvta_generic_to_shared(sm.tmp) + FSE_SLOTS * RING_STRIDE;
-    const bool tables_ok = sl.blk != NONE32 && sl.status == CZS_OK && sl.log[0] >= 0 && sl.log[1] >= 0 && sl.log[2] >= 0;
-    enum { BAR_EMPTY = 1, BAR_FULL = 3, BAR_SETUP = 5, BAR_FIN = 6 };
-    auto bar_sync = [](int id) { asm volatile("bar.sync %0, 64;" ::"r"(id) : "memory"); };
-    auto bar_arrive = [](int id) { asm volatile("bar.arrive %0, 64;" ::"r"(id) : "memory"); };
-    const uint32_t hand_base = (uint32_t)__cvta_generic_to_shared(&sm.hand[0][0][0]) + lane * 16u;
-    constexpr uint32_t HAND_VEC = FSE_SLOTS * 16u, HAND_BUF = 3u * HAND_VEC;
-    if (warp == 0) {
-        // ======== walker ========
-        RevBitsWin br;
-        bool go = tables_ok;
-        if (go) go = br.init(sl.bits, (int)sl.bits_len, ring_addr);
-        if (has) misc[lane] = go ? 1u : 0u;
-        const uint32_t n = go ? sl.n_seq : 0u;
-        uint32_t maxn = n;
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) maxn = max(maxn, __shfl_xor_sync(0xFFFFFFFFu, maxn, o));
-        const uint32_t logLL = go ? (uint32_t)sl.log[0] : 0u, logOF = go ? (uint32_t)sl.log[1] : 0u, logML = go ? (uint32_t)sl.log[2] : 0u;
-        const uint32_t mLL = (1u << logLL) - 1u, mOF = (1u << logOF) - 1u, mML = (1u << logML) - 1u;
-        const uint32_t ent = (uint32_t)__cvta_generic_to_shared(sm.entries);
-        uint32_t tLL = ent + 2u * sl.tbl[0], tOF = ent + 2u * sl.tbl[1], tML = ent + 2u * sl.tbl[2];  // byte addresses
-        asm volatile("" : "+r"(tLL), "+r"(tOF), "+r"(tML));  // opaque: keeps "base + 2 * index" one LEA instead of (table + index) * 2 + smem base
-        auto lds16 = [](uint32_t a) { uint32_t v; asm volatile("ld.volatile.shared.u16 %0, [%1];" : "=r"(v) : "r"(a) : "memory"); return v; };
-        uint32_t eLL = 0, eOF = 0, eML = 0;
-        if (go) {  // init order LL, OF, ML (:207-218)
-            eLL = lds16(tLL + 2u * br.get((int)logLL));
-            eOF = lds16(tOF + 2u * br.get((int)logOF));
-            eML = lds16(tML + 2u * br.get((int)logML));
-            cp_async_commit();
-            cp_async_wait<0>();
-            const uint4 top = *reinterpret_cast<const uint4*>(reinterpret_cast<const uint8_t*>(sm.tmp) + lane * RING_STRIDE + 16 + RevBitsWin::RING - 16);
-            *reinterpret_cast<uint4*>(reinterpret_cast<uint8_t*>(sm.tmp) + lane * RING_STRIDE) = top;  // the mirror starts out equal
-        }
-        __syncwarp();
-        bar_sync(BAR_SETUP);  // both warps hold their slots in registers: the slot array becomes the hand-over buffers
-        // 96 unread bits at P: x2 first.  Extra bits (<= 63) and the three state updates (<= 26) of one step all lie inside,
-        // so nothing on the chain waits for a ring read whose address depends on this step's codes.
-        uint32_t x0 = 0, x1 = 0, x2 = 0;
-        uint32_t rw0 = 0, rw1 = 0, rw2 = 0, rw3 = 0, rsh = 0;
-        // in two halves: the four ring reads go out as soon as the new P is known (before the next-state lookups, whose
-        // addresses take longer to form), the funnel shifts that consume them come after those lookups
-        auto window_issue = [&]() {
-            const uint32_t a = br.ring + (((uint32_t)br.P >> 3) & (RevBitsWin::RING - 4));
-            rsh = (uint32_t)br.P & 31u;
-            // the word holding bit P and the three below it (mirror: no wrap)
-            asm volatile("ld.volatile.shared.u32 %0, [%1];" : "=r"(rw3) : "r"(a) : "memory");
-            asm volatile("ld.volatile.shared.u32 %0, [%1+-4];" : "=r"(rw2) : "r"(a) : "memory");
-            asm volatile("ld.volatile.shared.u32 %0, [%1+-8];" : "=r"(rw1) : "r"(a) : "memory");
-            asm volatile("ld.volatile.shared.u32 %0, [%1+-12];" : "=r"(rw0) : "r"(a) : "memory");
-        };
-        auto window_finish = [&]() {
-            x2 = __funnelshift_r(rw2, rw3, rsh); x1 = __funnelshift_r(rw1, rw2, rsh); x0 = __funnelshift_r(rw0, rw1, rsh);
-        };
-        auto load_window = [&]() { window_issue(); window_finish(); };
-        // the ring's look-after with the mirror kept equal: the chunk that lands in the top slot lands below the ring as well
-        auto refill = [&](unsigned act) {
-            const int cn = (br.P - 1) >> 7;
-            const bool left = cn < br.chunk, need = left && br.chunk >= RevBitsWin::RING / 16;
-            const uint32_t slot = (uint32_t)br.chunk & (RevBitsWin::RING / 16 - 1);
-            const uint8_t* src = br.c_lo + (need ? ((br.chunk - RevBitsWin::RING / 16) << 4) : 0);
-            cp_async16_sz(need ? br.ring + (slot << 4) : dummy, src, need ? 16u : 0u);
-            const bool top = need && slot == RevBitsWin::RING / 16 - 1;
-            if (__any_sync(act, top)) cp_async16_sz(top ? br.ring - 16u : dummy, src, top ? 16u : 0u);  // one chunk in eight
-            br.chunk -= left ? 1 : 0;
-        };
-        uint32_t llb = 0, mlb = 0, nbLL = 0, nbML = 0, nbOF = 0;
-        auto prep = [&]() {  // what the next step needs from the entries just looked up
-            llb = sm.ll_code[fse_entry_sym(eLL)] >> 27; mlb = sm.ml_code[fse_entry_sym(eML)] >> 27;
-            nbLL = fse_entry_nbits(eLL, logLL); nbML = fse_entry_nbits(eML, logML); nbOF = fse_entry_nbits(eOF, logOF);
-        };
-        if (go) { load_window(); prep(); }
-        // one step: returns the three hand-over words; MORE = false is the last sequence (states are not updated, :258)
-        auto step = [&](auto more_tag, uint32_t& hx, uint32_t& lx, uint32_t& codes) {
-            constexpr bool MORE = decltype(more_tag)::value;
-            const uint32_t extras = (fse_entry_sym(eOF) & 31u) + mlb + llb;  // read in the order OF, ML, LL (:239)
-            hx = x2; lx = x1;
-            codes = __byte_perm(__byte_perm(eLL, eML, 0x0051), eOF, 0x7510);  // bytes: LL entry >> 8, ML entry >> 8, OF entry >> 8
-            if (MORE) {
-                br.P -= (int)(extras + nbLL + nbML + nbOF);
-                window_issue();  // x0..x2 keep this step's bits until window_finish()
-                // state bits (LL, ML, OF, :258-276) start `extras` bits into the window
-                const uint32_t za = __funnelshift_l(x1, x2, extras), zb = __funnelshift_l(x0, x1, extras);  // shift taken modulo 32
-                const uint32_t z = (extras & 32u) ? zb : za;
-                // next state = base_line + bits = ((next_state << nb) | top nb bits) without bit `log` and above
-                const uint32_t iLL = __funnelshift_l(z, eLL, nbLL) & mLL;
-                const uint32_t z1 = z << nbLL;
-                const uint32_t iML = __funnelshift_l(z1, eML, nbML) & mML;
-                const uint32_t z2 = z1 << nbML;
-                const uint32_t iOF = __funnelshift_l(z2, eOF, nbOF) & mOF;
-                eLL = lds16(tLL + 2u * iLL); eML = lds16(tML + 2u * iML); eOF = lds16(tOF + 2u * iOF);
-                window_finish();
-                prep();
-            } else {
-                br.P -= (int)extras;
-            }
-        };
-        const uint32_t n_batches = (maxn + FSE_HAND_STEPS - 1) / FSE_HAND_STEPS;
-        int p1 = 0x40000000, p2 = 0x40000000, p3 = 0x40000000;  // P at the start of the previous three batches ("far above": nothing may stay in flight yet)
-        for (uint32_t b = 0; b < n_batches; b++) {
-            const uint32_t i0 = b * FSE_HAND_STEPS, buf = b & 1u;
-            bar_sync(BAR_EMPTY + (int)buf);
-            const uint32_t hb = hand_base + buf * HAND_BUF;
-            if (i0 + FSE_HAND_STEPS < n) {  // four steps, none of them the last
-                // Ring: what this batch reads must have landed.  One commit group per batch; the group of batch j asked for chunks
-                // up to (head chunk at the start of j) - 8, and this batch reads no chunk below (head chunk now) - 4: a group
-                // may stay in flight while the head has moved less than four chunks since its batch began, which holds if it
-                // moved at most 384 bits.  Always true for the previous batch (<= 356 bits per batch); typical streams (~25
-                // bits per sequence) leave three groups, i.e. a dozen steps, for a request to come back from DRAM.
-                const unsigned act = __activemask();
-                if (__all_sync(act, p3 - br.P <= 384)) cp_async_wait<3>();
-                else if (__all_sync(act, p2 - br.P <= 384)) cp_async_wait<2>();
-                else cp_async_wait<1>();
-                p3 = p2; p2 = p1; p1 = br.P;
-                uint32_t w[12];
-                step(std::true_type{}, w[0], w[1], w[2]); step(std::true_type{}, w[3], w[4], w[5]);
-                step(std::true_type{}, w[6], w[7], w[8]); step(std::true_type{}, w[9], w[10], w[11]);
-                asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(hb), "r"(w[0]), "r"(w[1]), "r"(w[2]), "r"(w[3]) : "memory");
-                asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(hb + HAND_VEC), "r"(w[4]), "r"(w[5]), "r"(w[6]), "r"(w[7]) : "memory");
-                asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(hb + 2u * HAND_VEC), "r"(w[8]), "r"(w[9]), "r"(w[10]), "r"(w[11]) : "memory");
-                // four steps consume at most 356 bits, i.e. leave at most three 16-byte chunks behind
-                refill(act);
-                if (__any_sync(act, ((br.P - 1) >> 7) < br.chunk)) { refill(act); refill(act); }  // usually less than one chunk per batch
-                cp_async_commit();
-            } else if (i0 < n) {  // the block's last one to four steps
-                for (uint32_t k = 0; i0 + k < n; k++) {
-                    uint32_t hx, lx, codes;
-                    cp_async_wait<0>();
-                    if (i0 + k + 1 < n) step(std::true_type{}, hx, lx, codes); else step(std::false_type{}, hx, lx, codes);
-                    const uint32_t wi = 3u * k;
-                    const uint32_t a0 = hb + (wi >> 2) * HAND_VEC + (wi & 3u) * 4u, a1 = hb + ((wi + 1u) >> 2) * HAND_VEC + ((wi + 1u) & 3u) * 4u,
-                                   a2 = hb + ((wi + 2u) >> 2) * HAND_VEC + ((wi + 2u) & 3u) * 4u;
-                    asm volatile("st.shared.u32 [%0], %1;" ::"r"(a0), "r"(hx) : "memory");
-                    asm volatile("st.shared.u32 [%0], %1;" ::"r"(a1), "r"(lx) : "memory");
-                    asm volatile("st.shared.u32 [%0], %1;" ::"r"(a2), "r"(codes) : "memory");
-                    refill(__activemask());
-                    cp_async_commit();
-                }
-            }
-            __syncwarp();
-            bar_arrive(BAR_FULL + (int)buf);
-        }
-        cp_async_wait<0>();
-        // rem only ever decreases: one look tells whether it went negative on the way.  (A lane that is not `go` leaves its 0: the
-        // packer may not have read it yet -- with no batches at all nothing orders this write behind that read.)
-        if (go) misc[lane] = (uint32_t)br.rem();
-        __syncwarp();
-        bar_sync(BAR_FIN);
-        return;
-    }
-    // ======== packer ========
-    int32_t st = sl.status;
-    uint32_t h0, h1, h2;
-    if (sl.first_in_frame) { h0 = 1; h1 = 4; h2 = 8; }  // scratch.cairo:35
-    else { h0 = sym_enc(0); h1 = sym_enc(1); h2 = sym_enc(2); }
-    const uint32_t h_in0 = h0, h_in1 = h1, h_in2 = h2;
-    uint32_t ml_total = 0;
-    __syncwarp();
-    bar_sync(BAR_SETUP);
-    const bool go = has && misc[lane] != 0u;
-    bool fast_ok = false;
-    {
-        const uint32_t n = go ? sl.n_seq : 0u;
-        uint32_t maxn = n;
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) maxn = max(maxn, __shfl_xor_sync(0xFFFFFFFFu, maxn, o));
-        const uint32_t n_batches = (maxn + FSE_HAND_STEPS - 1) / FSE_HAND_STEPS;
-        Seq* out = sl.out;
-        uint32_t trouble = 0;  // bit 20 set <=> a code beyond the tables turned up (:235-237)
-        auto one = [&](uint32_t hx, uint32_t lx, uint32_t codes) -> Seq {
-            // codes: the high bytes (symbol << 2 | two state bits) of the LL, ML and OF entries
-            const uint32_t ofc = (codes >> 18) & 63u;
-            const uint32_t lle = sm.ll_code[(codes >> 2) & 63u], mle = sm.ml_code[(codes >> 10) & 63u];
-            trouble |= (ofc << 15) | lle | mle;  // ofc >= 32 puts its bit 5 at bit 20
-            const uint32_t llb = lle >> 27, mlb = mle >> 27, ofb = ofc & 31u;
-            const uint32_t ofv = shr_clamp(hx, 32u - ofb);
-            const uint32_t y = __funnelshift_l(lx, hx, ofb);
-            const uint32_t mlv = shr_clamp(y, 32u - mlb), llv = shr_clamp(y << mlb, 32u - llb);
-            const uint32_t ll = (lle & 0xFFFFFu) + llv, ml = (mle & 0xFFFFFu) + mlv;
-            const uint32_t v = (1u << ofb) + ofv;  // :243
-            // do_offset_history (sequence_execution.cairo:85-129) with selects only:
-            // idx 0,1,2 = history slot, 3 = h0 - 1 (reachable only when ll == 0)
-            const uint32_t idx = v - (ll != 0);
-            const bool rep = v <= 3;
-            uint32_t cand = h0 - 1u;
-            cand = idx == 2 ? h2 : cand;
-            cand = idx == 1 ? h1 : cand;
-            cand = idx == 0 ? h0 : cand;
-            const uint32_t nz = min(v - 3u, REAL_OFF_CLAMP);
-            const uint32_t act = rep ? cand : nz;
-            h2 = (rep & (idx <= 1)) ? h2 : h1;
-            h1 = (rep & (idx == 0)) ? h1 : h0;
-            h0 = act;
-            ml_total += ml;  // the block's output size is regen + sum(ml): what czb_frame_sizes_* reports without executing
-            return (Seq)ll | ((Seq)ml << 17) | ((Seq)off29_pack(act) << 35);
-        };
-        bar_arrive(BAR_EMPTY); bar_arrive(BAR_EMPTY + 1);
-        for (uint32_t b = 0; b < n_batches; b++) {
-            const uint32_t i0 = b * FSE_HAND_STEPS, buf = b & 1u;
-            bar_sync(BAR_FULL + (int)buf);
-            const uint32_t hb = hand_base + buf * HAND_BUF;
-            if (i0 < n) {
-                uint32_t w[12];
-                asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(w[0]), "=r"(w[1]), "=r"(w[2]), "=r"(w[3]) : "r"(hb) : "memory");
-                asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(w[4]), "=r"(w[5]), "=r"(w[6]), "=r"(w[7]) : "r"(hb + HAND_VEC) : "memory");
-                asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(w[8]), "=r"(w[9]), "=r"(w[10]), "=r"(w[11]) : "r"(hb + 2u * HAND_VEC) : "memory");
-                if (i0 + FSE_HAND_STEPS <= n) {
-                    // four records leave as two 16-byte stores: a block's slice of the scratch is 32-byte aligned (k_fill_blocks)
-                    const Seq r0 = one(w[0], w[1], w[2]), r1 = one(w[3], w[4], w[5]), r2 = one(w[6], w[7], w[8]), r3 = one(w[9], w[10], w[11]);
-                    uint4* o4 = reinterpret_cast<uint4*>(out + i0);
-                    __stcs(o4, make_uint4((uint32_t)r0, (uint32_t)(r0 >> 32), (uint32_t)r1, (uint32_t)(r1 >> 32)));
-                    __stcs(o4 + 1, make_uint4((uint32_t)r2, (uint32_t)(r2 >> 32), (uint32_t)r3, (uint32_t)(r3 >> 32)));
-                } else {
-                    __stcs(out + i0, one(w[0], w[1], w[2]));
-                    if (i0 + 1 < n) __stcs(out + i0 + 1, one(w[3], w[4], w[5]));
-                    if (i0 + 2 < n) __stcs(out + i0 + 2, one(w[6], w[7], w[8]));
-                }
-            }
-            __syncwarp();
-            if (b + 2 < n_batches) bar_arrive(BAR_EMPTY + (int)buf);
-        }
-        __syncwarp();
-        bar_sync(BAR_FIN);
-        if (go) {
-            const int rem = (int)misc[lane];
-            if (!(trouble & FSE_BAD_CODE) && rem >= 0) { fast_ok = true; st = rem > 0 ? CZS_SEQ_EXTRA_BITS : CZS_OK; }  // :292-296
-        }
-    }
-    if (sl.blk == NONE32) return;
-#else
     if (warp != 0) return;  // (rotating the decode warp over the CTAs of an SM was measured: 28.3 -> 33.4 ms; the hardware already spreads them over the schedulers)
 
     // ---- phase 2: lane = block ----
@@ -477,14 +214,11 @@ __global__ void __launch_bounds__(FSE_WARPS * 32, 3) k_fse(const czb_frame_desc*
     else { h0 = sym_enc(0); h1 = sym_enc(1); h2 = sym_enc(2); }
     const uint32_t h_in0 = h0, h_in1 = h1, h_in2 = h2;
     uint32_t ml_total = 0;
-#endif
-    // The decode loop exists twice.  The fast form only notes THAT something went wrong (two ORs per step); a block for
-    // which it did is decoded again by the exact form, which records WHICH error came first, in the reference's order
-    // (two compares and selects per step: 8 % of the kernel when it was always on).
-    auto decode = [&](auto exact_tag) -> int32_t {
-    constexpr bool EXACT = decltype(exact_tag)::value;
+    // The decode loop exists twice.  The fast form (decode_lean, below) only notes THAT something went wrong; a block for
+    // which it did, or which it does not take, is decoded again by this exact form, which records WHICH error came first,
+    // in the reference's order (two compares and selects per step: 8 % of the kernel when it was always on).
+    auto decode = [&]() -> int32_t {
     int32_t st = CZS_OK;
-    uint32_t trouble = 0;  // fast form: bit 20 set <=> a bad code or an over-read happened somewhere
     h0 = h_in0; h1 = h_in1; h2 = h_in2;
     ml_total = 0;
     {
@@ -526,13 +260,9 @@ __global__ void __launch_bounds__(FSE_WARPS * 32, 3) k_fse(const czb_frame_desc*
                 br.step_sync();
                 const uint32_t ofc = fse_entry_sym(eOF);
                 // :235-237; codes beyond the tables give (0,255) -> TooManyBits
-                if (EXACT) {
-                    const bool bad_code = ((ofc >> 5) | (((lle | mle) >> 20) & 1u)) != 0;
-                    const int32_t code_status = ofc >= 32 ? CZS_SEQ_UNSUPPORTED_OFFSET : CZS_SEQ_GET_BITS_ERROR;
-                    st = (st == CZS_OK && bad_code) ? code_status : st;
-                } else {
-                    trouble |= (ofc << 15) | lle | mle;  // ofc >= 32 puts its bit 5 at bit 20
-                }
+                const bool bad_code = ((ofc >> 5) | (((lle | mle) >> 20) & 1u)) != 0;
+                const int32_t code_status = ofc >= 32 ? CZS_SEQ_UNSUPPORTED_OFFSET : CZS_SEQ_GET_BITS_ERROR;
+                st = (st == CZS_OK && bad_code) ? code_status : st;
                 const uint32_t llb = lle >> 27, mlb = mle >> 27, ofb = ofc & 31u;
                 const uint32_t extras = ofb + mlb + llb;  // <= 63 bits, read in the order OF, ML, LL (:239)
                 // The three state updates (LL, ML, OF, <= 26 bits, :258-276) come from their own 32-bit window below the
@@ -583,8 +313,7 @@ __global__ void __launch_bounds__(FSE_WARPS * 32, 3) k_fse(const czb_frame_desc*
                     nbLL = fse_entry_nbits(eLL, logLL); nbML = fse_entry_nbits(eML, logML); nbOF = fse_entry_nbits(eOF, logOF);
                 }
                 // :281-283; the no-RLE variant traps on the unwrap at :279 instead
-                if (EXACT) st = (st == CZS_OK && br.rem() < 0) ? short_status : st;
-                // (fast form: rem only ever decreases, so one look after the loop tells whether it went negative on the way)
+                st = (st == CZS_OK && br.rem() < 0) ? short_status : st;
             };
             // Four steps consume at most 356 bits, i.e. leave at most three 16-byte chunks behind: the ring is looked after
             // once per four steps (three always-issued cp.async) instead of once per step.
@@ -593,26 +322,19 @@ __global__ void __launch_bounds__(FSE_WARPS * 32, 3) k_fse(const czb_frame_desc*
             using Q3 = std::integral_constant<int, 3>; using QN = std::integral_constant<int, -1>;
             uint32_t i = 0;
             for (; i + 4 < n_seq; i += 4) {
-#if CZB_FSE_QUAD
                 step(i, std::true_type{}, R0{}, Q0{}); step(i + 1, std::true_type{}, R0{}, Q1{});
                 step(i + 2, std::true_type{}, R0{}, Q2{}); step(i + 3, std::true_type{}, R3{}, Q3{});
                 uint4* o4 = reinterpret_cast<uint4*>(out + i);
                 __stcs(o4, make_uint4((uint32_t)quad[0], (uint32_t)(quad[0] >> 32), (uint32_t)quad[1], (uint32_t)(quad[1] >> 32)));
                 __stcs(o4 + 1, make_uint4((uint32_t)quad[2], (uint32_t)(quad[2] >> 32), (uint32_t)quad[3], (uint32_t)(quad[3] >> 32)));
-#else
-                step(i, std::true_type{}, R0{}, QN{}); step(i + 1, std::true_type{}, R0{}, QN{});
-                step(i + 2, std::true_type{}, R0{}, QN{}); step(i + 3, std::true_type{}, R3{}, QN{});
-#endif
             }
             for (; i + 1 < n_seq; i++) step(i, std::true_type{}, R1{}, QN{});
             step(i, std::false_type{}, R0{}, QN{});
-            if (!EXACT && ((trouble & FSE_BAD_CODE) || br.rem() < 0)) st = CZS_NOT_DECODED;  // placeholder: the exact form decides
             if (st == CZS_OK && br.rem() > 0) st = CZS_SEQ_EXTRA_BITS;  // :292-296
         }
     }
     return st;
     };
-#if CZB_FSE_SPLIT == 0
     // The fast form, one warp, written for instruction count.  ALU instructions issue at one per two cycles per scheduler
     // and the decode warp is alone on its scheduler, so a step costs ~1.6 cycles per instruction whatever the dependency
     // chain looks like (154 instructions and ~250 cycles in the round-1 form; splitting the step over two warps left the
@@ -771,22 +493,12 @@ __global__ void __launch_bounds__(FSE_WARPS * 32, 3) k_fse(const czb_frame_desc*
         if (br.rem() < 0) return CZS_NOT_DECODED;  // placeholder: the exact form decides
         return br.rem() > 0 ? CZS_SEQ_EXTRA_BITS : CZS_OK;  // :292-296
     };
-#endif
-#if CZB_FSE_SPLIT == 1
-    if (st == CZS_OK && !fast_ok) st = decode(std::true_type{});  // the exact loop: which error came first, in the reference's order
-#elif CZB_FSE_SPLIT == 0
     if (st == CZS_OK) {
         const unsigned decoders = __activemask();
         st = decode_lean();
         __syncwarp(decoders);  // the exact loop lays its rings over the same scratch
-        if (st == CZS_NOT_DECODED) st = decode(std::true_type{});
+        if (st == CZS_NOT_DECODED) st = decode();
     }
-#else
-    if (st == CZS_OK) {
-        st = decode(std::false_type{});
-        if (st == CZS_NOT_DECODED) st = decode(std::true_type{});
-    }
-#endif
     BlockDesc& d = blocks[sl.blk];
     d.fse_status = st;
     d.hist_out[0] = h0; d.hist_out[1] = h1; d.hist_out[2] = h2;
