@@ -11,6 +11,7 @@ from .api import (  # noqa: F401
     CzbError,
     FrameDesc,
     FrameResult,
+    MAX_FRAME_OUTPUT,
     STATUS_NAMES,
     find_frame_end,
     frame_header_info,

@@ -8,6 +8,7 @@ _LIB_PATH = os.environ.get("CZB_LIB") or os.path.join(_HERE, "libcairo_zstd_b200
 _INCLUDE = os.path.join(os.path.dirname(_HERE), "include")
 
 FLAG_VERIFY_CHECKSUM = 1
+MAX_FRAME_OUTPUT = (1 << 31) - 1  # CZB_MAX_FRAME_OUTPUT: larger frames get CZS_UNSUPPORTED (CZS_DST_TOO_SMALL below that dst_cap)
 
 
 class CzbError(RuntimeError):

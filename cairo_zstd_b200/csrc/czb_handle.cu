@@ -129,7 +129,7 @@ static int fd_run_device(czb_frame_decoder* fd) {
         pos += 3 + pb.content;
         if (pb.last) break;
     }
-    if (fd->hdr.fcs_bytes && fd->hdr.fcs > bound && fd->hdr.fcs < MAX_FRAME_OUT) bound = fd->hdr.fcs;
+    if (fd->hdr.fcs_bytes && fd->hdr.fcs > bound && fd->hdr.fcs <= MAX_FRAME_OUT) bound = fd->hdr.fcs;
     uint64_t cap = bound + 64;
     // source: only the bytes that arrived since the last run travel to the device
     if (n + 64 > fd->d_src_cap) {

@@ -55,7 +55,8 @@ static_assert(BIG_WIN_REACH >= (2 * BIG_WARPS_MAX - 1) * (int)EXEC_TILE, "bytes 
 struct WinView {
     uint8_t* win;     // BIG_WIN bytes of shared memory, 16-byte aligned
     uint8_t* obase;   // dst address of chunk-relative position 0
-    uint32_t gb;      // low 32 bits of obase: window index of position x is (gb + x) & BIG_WIN_MASK
+    uint32_t gb;      // low 32 bits of obase: window index of position x is (gb + x) & BIG_WIN_MASK (exact across a wrap of
+                      // the 32-bit sum, BIG_WIN divides 2^32; x is chunk-relative and the frame position does not enter it)
     int lo_rel;       // positions >= lo_rel are in the window, older ones only in dst
     __device__ __forceinline__ uint32_t idx(int x) const { return (gb + (uint32_t)x) & BIG_WIN_MASK; }
     __device__ __forceinline__ uint8_t rd(int x) const { return x >= lo_rel ? win[idx(x)] : __ldcg(obase + x); }
@@ -229,15 +230,18 @@ __global__ void __launch_bounds__(EXEC_WARPS * 32, EXEC_MIN_CTAS) k_exec(const c
                 const uint32_t lit_used = __shfl_sync(0xFFFFFFFFu, lsum, 31);
                 // Errors are rare: one cheap test that is exact for "some lane fails" (totals for the literal and
                 // capacity checks, one unsigned compare per lane for offset 0 / offset beyond the output so far;
-                // out <= cap < 2^28, so 32 bits suffice), then the reference's checks in its order only if it fires.
+                // out <= cap < 2^31 and a chunk spans < 2^25, so 32 bits suffice; one more for a possibly far offset,
+                // see off29_far), then the reference's checks in its order only if it fires.
                 const uint32_t before_match32 = (uint32_t)out + my_out + ll;
-                const bool suspicious = (uint64_t)lit_pos + lit_used > n_lit || out + span > cap || (have && off - 1u >= before_match32);
+                const bool suspicious = (uint64_t)lit_pos + lit_used > n_lit || out + span > cap || (have && (off - 1u >= before_match32 || off == OFF29_CLAMP));
                 if (__any_sync(0xFFFFFFFFu, suspicious)) {
                     const uint64_t before_match = out + my_out + ll;  // DecodeBuffer.len() when repeat() is called
                     int32_t err = CZS_OK;
                     if (have) {
                         if (ll > 0 && (uint64_t)my_lit + ll > n_lit) err = CZS_EXEC_NOT_ENOUGH_BYTES_FOR_SEQUENCE;  // :29-37
                         else if (off == 0) err = CZS_EXEC_ZERO_OFFSET;                                            // :47-49
+                        else if (ml > 0 && off == OFF29_CLAMP && off29_far(seq_off29(seqs[i]), before_match))     // the raw field, not the resolved offset
+                            err = CZS_UNSUPPORTED;
                         else if (ml > 0 && off > before_match)                                                      // decode_buffer.cairo:65-93
                             err = (before_match <= fi.window) ? CZS_NOT_ENOUGH_BYTES_IN_DICTIONARY : CZS_OFFSET_TOO_BIG;
                         else if (before_match + ml > cap) err = cap_status;
@@ -250,7 +254,8 @@ __global__ void __launch_bounds__(EXEC_WARPS * 32, EXEC_MIN_CTAS) k_exec(const c
                     out += span; lit_pos += lit_used;
                     continue;
                 }
-                // general path (long segments): publish the 64 segments of this chunk
+                // general path (long segments): publish the 64 segments of this chunk.  The checks passed, so
+                // off <= before_match <= cap < 2^31 and positions are chunk-relative (< 2^25): the int casts below hold.
                 const uint32_t segA = my_out, segM = my_out + ll;
                 sm.bound[2 * lane] = segA; sm.bound[2 * lane + 1] = segM;
                 sm.segdelta[2 * lane] = (int)my_lit - (int)segA;
@@ -587,6 +592,8 @@ __global__ void __launch_bounds__(BIG_WARPS * 32, BIG_MIN_CTAS) k_exec_big(const
                 if (have) {
                     if (ll > 0 && (uint64_t)my_lit + ll > n_lit) err = CZS_EXEC_NOT_ENOUGH_BYTES_FOR_SEQUENCE;  // :29-37
                     else if (off == 0) err = CZS_EXEC_ZERO_OFFSET;                                            // :47-49
+                    else if (ml > 0 && off == OFF29_CLAMP && off29_far(seq_off29(seqs[i]), before_match))     // the raw field, not the resolved offset
+                        err = CZS_UNSUPPORTED;
                     else if (ml > 0 && off > before_match)                                                      // decode_buffer.cairo:65-93
                         err = (before_match <= fi.window) ? CZS_NOT_ENOUGH_BYTES_IN_DICTIONARY : CZS_OFFSET_TOO_BIG;
                     else if (before_match + ml > cap) err = cap_status;

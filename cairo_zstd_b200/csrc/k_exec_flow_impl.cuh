@@ -210,13 +210,16 @@ __global__ void __launch_bounds__(FLOW_WARPS * 32, FLOW_P_MIN_CTAS) k_exec_flow(
                 for (uint32_t i = threadIdx.x; i < FLOW_BITWORDS; i += FLOW_WARPS * 32) sm.ready[i] = 0u;
                 for (uint32_t i = threadIdx.x; i < FLOW_NSLOT; i += FLOW_WARPS * 32) sm.done[i] = 0u;
                 __syncthreads();
-                const uint32_t batch_out0 = (uint32_t)(out + out_total);  // frame position of the batch's first byte (< 2^28)
+                const uint32_t batch_out0 = (uint32_t)(out + out_total);  // frame position of the batch's first byte (<= cap < 2^31)
                 if (warp == 0) {
                     // 64-bit running totals, stored saturated: a malformed block whose lengths add up to more than 2^31 must
-                    // fail its capacity / literal checks, not wrap around them
+                    // fail its capacity / literal checks, not wrap around them.  Output offsets saturate where the frame position
+                    // reaches 2^31 (> cap), so that position + chunk span (< 2^25) stays below 2^32 in the chunks' u32 sums.
                     unsigned long long cl = 0, co = 0;
                     uint32_t last_long = 0xFFFFu;
                     auto sat = [](unsigned long long v) -> uint32_t { return v < 0x7FFFFFFFull ? (uint32_t)v : 0x7FFFFFFFu; };
+                    const unsigned long long out_lim = 0x80000000ull - batch_out0;
+                    auto sat_out = [out_lim](unsigned long long v) -> uint32_t { return (uint32_t)(v < out_lim ? v : out_lim); };
                     for (uint32_t b = 0; b < nb; b += 32) {
                         const uint32_t c = b + lane;
                         const uint32_t vl = c < nb ? sm.chunk_lit[c] : 0u, vo = c < nb ? sm.chunk_out[c] : 0u;
@@ -230,11 +233,11 @@ __global__ void __launch_bounds__(FLOW_WARPS * 32, FLOW_P_MIN_CTAS) k_exec_flow(
                             const uint32_t a = __shfl_up_sync(0xFFFFFFFFu, il, o), b2 = __shfl_up_sync(0xFFFFFFFFu, io, o);
                             if ((int)lane >= o) { il += a; io += b2; }
                         }
-                        if (c < nb) { sm.chunk_lit[c] = sat(cl + il - vl); sm.chunk_out[c] = sat(co + io - vo); }
+                        if (c < nb) { sm.chunk_lit[c] = sat(cl + il - vl); sm.chunk_out[c] = sat_out(co + io - vo); }
                         cl += __shfl_sync(0xFFFFFFFFu, il, 31); co += __shfl_sync(0xFFFFFFFFu, io, 31);
                     }
                     if (lane == 0) {
-                        sm.chunk_lit[nb] = sat(cl); sm.chunk_out[nb] = sat(co);
+                        sm.chunk_lit[nb] = sat(cl); sm.chunk_out[nb] = sat_out(co);
                         sm.next_chunk = 0; sm.head = 0; sm.retired_out = batch_out0; sm.win_lo = batch_out0;
                         sm.err_chunk = NONE32; sm.err_status = CZS_OK; sm.abort = 0u;
                     }
@@ -272,6 +275,8 @@ __global__ void __launch_bounds__(FLOW_WARPS * 32, FLOW_P_MIN_CTAS) k_exec_flow(
                     if (have) {
                         if (ll > 0 && (uint64_t)my_lit + ll > n_lit) err = CZS_EXEC_NOT_ENOUGH_BYTES_FOR_SEQUENCE;  // :29-37
                         else if (off == 0) err = CZS_EXEC_ZERO_OFFSET;                                            // :47-49
+                        else if (ml > 0 && off == OFF29_CLAMP && off29_far(seq_off29(rec), segM))                // the raw field, not the resolved offset
+                            err = CZS_UNSUPPORTED;
                         else if (ml > 0 && off > segM)                                                              // decode_buffer.cairo:65-93
                             err = ((uint64_t)segM <= fi.window) ? CZS_NOT_ENOUGH_BYTES_IN_DICTIONARY : CZS_OFFSET_TOO_BIG;
                         else if ((uint64_t)segM + ml > cap) err = cap_status;

@@ -7,7 +7,8 @@
 //
 // XXH64 has exactly four independent accumulators per 32-byte stripe, so a frame gets four
 // lanes (lane k owns accumulator v_{k+1}); a warp hashes 8 frames at once and every load
-// instruction reads whole 32-byte sectors.  HBM-bound streaming read of the decoded bytes.
+// instruction reads whole 32-byte sectors.  HBM-bound streaming read of the decoded bytes.  Lengths and stripe indices are
+// 64-bit: any frame size.  A frame of MAX_FRAME_OUT bytes is 2^26 stripes on four lanes.
 #include "czb_internal.cuh"
 
 namespace czb {

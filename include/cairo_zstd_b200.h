@@ -22,8 +22,15 @@
  *   1. Direct 4-bit Huffman weights are read in RFC 8878 order (even index = high nibble).
  *      src/huff0/huff0_decoder.cairo:302 reads `idx | 1 == 1`, i.e. (idx|1)==1; the reference's
  *      own fixtures pin only the RFC behaviour (DESIGN.md section 2).
- *   2. CZS_UNSUPPORTED marks input the reference accepts but this build does not decode:
- *      frames whose output reaches 2^28 - 1 bytes.  It never means "malformed".
+ *   2. CZS_UNSUPPORTED marks input this build does not decode:
+ *      a. frames whose output exceeds CZB_MAX_FRAME_OUTPUT (2^31 - 1) bytes, when dst_cap is at least that
+ *         (with a smaller dst_cap the frame fails with CZS_DST_TOO_SMALL, as any frame that overflows dst);
+ *      b. a sequence with a directly coded offset of 2^28 - 1 or more whose match starts at output position
+ *         2^28 - 1 or later: the decoded sequence keeps 28 bits of such an offset.  The status replaces the
+ *         reference's offset check (CZS_OFFSET_TOO_BIG / CZS_NOT_ENOUGH_BYTES_IN_DICTIONARY) in its order,
+ *         after the literal-length check and before the capacity check, so the frame may also be malformed.
+ *         A repeat code that takes such an offset from an earlier block's history resolves it exactly, and
+ *         a far offset whose match starts below 2^28 - 1 exceeds the output so far: the reference's status.
  *      (Huffman-weight FSE tables with an accuracy log above 9 -- the reference passes a limit of
  *      100, huff0_decoder.cairo:176 -- are decoded: tests/test_gpu_fuzz.py.)
  */
@@ -39,6 +46,10 @@ extern "C" {
 #endif
 
 #define CZB_ABI_VERSION 1
+
+/* Largest decoded size of one frame this build decodes (bytes).  Size dst spans and route larger frames elsewhere:
+ * a frame with more output gets CZS_UNSUPPORTED (or CZS_DST_TOO_SMALL when dst_cap is below this). */
+#define CZB_MAX_FRAME_OUTPUT 0x7FFFFFFFull
 
 /* One frame of a batch: the reference's `ref source: @ByteArraySlice` (borrowed, immutable,
  * src/utils/byte_array.cairo:9-13) plus the caller-owned span that receives what

@@ -109,9 +109,12 @@ typedef enum czs_status {
 
     /* Boundary-only codes (no reference counterpart) */
     CZS_DST_TOO_SMALL = 102,   /* caller's output span cannot hold the frame */
-    CZS_UNSUPPORTED = 103,     /* NOT malformed input: accepted by the reference but outside this
-                                  build's limit (DESIGN.md "Limits"): a frame whose output reaches
-                                  2^28 - 1 bytes (sequence records keep a 28-bit offset) */
+    CZS_UNSUPPORTED = 103,     /* outside this build's limits (DESIGN.md "Limits"): a frame whose
+                                  output exceeds CZB_MAX_FRAME_OUTPUT (2^31 - 1) bytes, or a direct
+                                  offset of 2^28 - 1 or more whose match starts at output position
+                                  2^28 - 1 or later (sequence records keep 28 bits of such an offset).
+                                  The second case is reported where the reference checks the offset,
+                                  whether the offset is valid or not: the frame may be malformed too */
     CZS_CUDA_ERROR = 104,      /* CUDA runtime failure; see czb_last_error() */
     CZS_BAD_ARGUMENT = 105,
     CZS_NOT_DECODED = 106      /* result slot never written (internal) */
