@@ -89,7 +89,8 @@ class Rle:
 
 @dataclass
 class Seqs:
-    """A compressed block.  literals: bytes (Raw literals section) or ("rle", byte, n).  seqs: [(ll, ml, ofv)].
+    """A compressed block.  literals: bytes (Raw literals section), ("rle", byte, n) or a Huffman section spec
+    (tests/hufbuild.py: Huf, Treeless).  seqs: [(ll, ml, ofv)].
     tables: (LL, OF, ML) specs.  nbseq_form: 1, 2 or 3 forces that number-of-sequences header form."""
     literals: object
     seqs: list
@@ -101,7 +102,7 @@ def _lit_bytes(lits):
     if isinstance(lits, tuple):
         assert lits[0] == "rle"
         return bytes([lits[1]]) * lits[2]
-    return bytes(lits)
+    return bytes(getattr(lits, "data", lits))
 
 
 # ---------------------------------------------------------------------------
@@ -283,10 +284,13 @@ def _nbseq_header(n, form):
     return bytes([255]) + struct.pack("<H", n - 0x7F00)
 
 
-def encode_seqs_block(b, prev):
-    """Body of one compressed block; `prev` = the (LL, OF, ML) streams of the last block that had sequences (for "repeat")."""
+def encode_seqs_block(b, prev, lit_state=None):
+    """Body of one compressed block; `prev` = the (LL, OF, ML) streams of the last block that had sequences (for "repeat");
+    `lit_state` = what the frame's Huffman sections so far left behind (the tree a Treeless section reuses)."""
     if isinstance(b.literals, tuple):
         lit = _lit_header(1, b.literals[2]) + bytes([b.literals[1]])
+    elif hasattr(b.literals, "section"):
+        lit = b.literals.section({} if lit_state is None else lit_state)
     else:
         lit = _lit_header(0, len(b.literals)) + bytes(b.literals)
     n = len(b.seqs)
@@ -346,6 +350,7 @@ def build_frame(blocks, single_segment=True, window_log=None, fcs_width=None, ch
         hdr += struct.pack("<Q", fcs)
     body = b""
     prev = None
+    lit_state = {}
     for i, b in enumerate(blocks):
         last = int(i == len(blocks) - 1)
         if isinstance(b, Raw):
@@ -353,7 +358,7 @@ def build_frame(blocks, single_segment=True, window_log=None, fcs_width=None, ch
         elif isinstance(b, Rle):
             body += _block_header(last, 1, b.n) + bytes([b.byte])
         else:
-            blk, prev = encode_seqs_block(b, prev)
+            blk, prev = encode_seqs_block(b, prev, lit_state)
             if body_hook:
                 blk = body_hook(i, blk)
             assert len(blk) <= BLOCK_MAX
