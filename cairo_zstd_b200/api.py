@@ -58,6 +58,11 @@ class DebugBlock(C.Structure):
     ]
 
 
+class DebugWaveTotals(C.Structure):
+    _fields_ = [("n_blocks", C.c_uint64), ("lit_bytes", C.c_uint64), ("n_seq", C.c_uint64), ("n_huf", C.c_uint64),
+                ("n_fse", C.c_uint64), ("src_bytes", C.c_uint64), ("frame_cls", C.c_uint32 * 32), ("fse_cls", C.c_uint32 * 32)]
+
+
 def _parse_status_names():
     names = {}
     try:
@@ -86,7 +91,7 @@ EXPORTS = [
     "czb_debug_last_wave_counts", "czb_debug_copy_blocks", "czb_debug_copy_literals", "czb_debug_copy_sequences",
     "czb_kernel_launches", "czb_profile_enable", "czb_profile_collect", "czs_status_name",
     "czb_split_frames_host", "czb_split_frames_device", "czb_frame_sizes_device", "czb_frame_sizes_host",
-    "czb_dictionary_parse_host", "czb_plan_batch_device", "czb_plan_destroy", "czb_decode_batch_device_planned", "czb_debug_fd_device_work", "czb_debug_guard_faults", "czb_debug_flow_watchdog", "czb_partition_frames", "czb_multi_create", "czb_multi_destroy", "czb_decode_batch_multi", "czb_multi_last_error",
+    "czb_dictionary_parse_host", "czb_plan_batch_device", "czb_plan_destroy", "czb_decode_batch_device_planned", "czb_debug_fd_device_work", "czb_debug_guard_faults", "czb_debug_flow_watchdog", "czb_debug_plan_waves", "czb_partition_frames", "czb_multi_create", "czb_multi_destroy", "czb_decode_batch_multi", "czb_multi_last_error",
 ]
 
 _lib = None
@@ -147,6 +152,7 @@ def load_library():
     L.czb_debug_fd_device_work.argtypes = [vp, P(u64), P(u64)]
     L.czb_debug_flow_watchdog.argtypes = [P(u32)]
     L.czb_debug_guard_faults.argtypes = [vp, P(u64)]
+    L.czb_debug_plan_waves.argtypes = [vp, P(u64), P(u64), P(DebugWaveTotals), u64]
     L.czb_split_frames_host.argtypes = [C.c_char_p, u64, P(FrameSpan), u64, P(u64), P(u64), P(u64)]
     L.czb_split_frames_device.argtypes = [vp, vp, u64, vp, u64, vp, vp]
     L.czb_frame_sizes_device.argtypes = [vp, vp, vp, u64, vp]
@@ -358,6 +364,14 @@ class Context:
         return {k: (ms[i], n[i]) for i, k in enumerate(self.KERNEL_CLASSES) if n[i]}
 
     # ---- debug taps ----
+    def plan_waves(self, plan):
+        """czb_debug_plan_waves: (frames per wave, [DebugWaveTotals] of every wave) of a plan from plan_batch_device."""
+        w, nw = C.c_uint64(), C.c_uint64()
+        self._check(self._L.czb_debug_plan_waves(plan, C.byref(w), C.byref(nw), None, 0))
+        out = (DebugWaveTotals * max(nw.value, 1))()
+        self._check(self._L.czb_debug_plan_waves(plan, None, None, out, nw.value))
+        return w.value, [out[i] for i in range(nw.value)]
+
     def debug_last_wave(self):
         nb, lb, ns = C.c_uint64(), C.c_uint64(), C.c_uint64()
         self._L.czb_debug_last_wave_counts(self._h, C.byref(nb), C.byref(lb), C.byref(ns))

@@ -241,22 +241,18 @@ static int decode_batch_impl(czb_context* ctx, const czb_frame_desc* descs, czb_
     uint64_t W = std::min<uint64_t>((n + 127) / 128 * 128, ctx->wave_frames);
     while ((n + W - 1) / W > kMaxWaves) W *= 2;
     uint64_t n_waves = 0;
-    bool exact_classes = true;  // per-section size classes come from the scan; a planning retry only has per-frame data
     const WaveTotals* totals_host = ctx->totals_h;
     if (plan) {  // scan with the planned wave size (device-side totals and size classes for k_fill_blocks), no read-back
         W = plan->W; n_waves = plan->n_waves; totals_host = plan->totals.data();
         CZB_CUDA(ctx, cudaMemsetAsync(ctx->totals_d.p, 0, n_waves * sizeof(WaveTotals), stream));
         { ProfScope ps(ctx, stream, 0); launch_scan_frames(lc, descs, ctx->infos.p, n, W, ctx->totals_d.p, resume); }
     }
-    for (int attempt = 0; !plan; attempt++) {
-        exact_classes = attempt == 0;
+    // A retry (a wave's scratch over the budget) scans again with the smaller wave size: the scan is the only code that
+    // produces wave totals, so a retried wave's totals are the ones a call starting at that wave size would see.
+    while (!plan) {
         n_waves = (n + W - 1) / W;
-        if (attempt == 0) {
-            CZB_CUDA(ctx, cudaMemsetAsync(ctx->totals_d.p, 0, n_waves * sizeof(WaveTotals), stream));
-            { ProfScope ps(ctx, stream, 0); launch_scan_frames(lc, descs, ctx->infos.p, n, W, ctx->totals_d.p, resume); }
-        } else {
-            launch_wave_totals(lc, ctx->infos.p, n, W, ctx->totals_d.p, n_waves);
-        }
+        CZB_CUDA(ctx, cudaMemsetAsync(ctx->totals_d.p, 0, n_waves * sizeof(WaveTotals), stream));
+        { ProfScope ps(ctx, stream, 0); launch_scan_frames(lc, descs, ctx->infos.p, n, W, ctx->totals_d.p, resume); }
         launch_publish_totals(lc, ctx->totals_d.p, ctx->totals_h_dev, n_waves);
         CZB_CUDA(ctx, cudaStreamSynchronize(stream));
         uint64_t worst = 0;
@@ -264,7 +260,7 @@ static int decode_batch_impl(czb_context* ctx, const czb_frame_desc* descs, czb_
         if ((ctx->no_overlap ? 1 : 2) * worst <= ctx->budget || W <= 128 || (n + W / 2 - 1) / (W / 2) > kMaxWaves) break;
         W = std::max<uint64_t>(128, (W / 2 + 127) / 128 * 128);
     }
-    if (plan_out) {  // keep a final scan with the final wave size consistent: a retry recomputed totals from per-frame data
+    if (plan_out) {
         plan_out->n = n; plan_out->W = W; plan_out->n_waves = n_waves;
         plan_out->totals.assign(ctx->totals_h, ctx->totals_h + n_waves);
     }
@@ -338,7 +334,7 @@ static int decode_batch_impl(czb_context* ctx, const czb_frame_desc* descs, czb_
             CZB_CUDA(ctx, cudaMemsetAsync(reinterpret_cast<uint8_t*>(ctx->blocks[s].p + t.n_blocks), kGuardByte, kGuardBytes, stream));
         }
         CZB_CUDA(ctx, cudaMemsetAsync(ctx->counters[s].p, 0, sizeof(WaveCounters), stream));
-        { ProfScope ps(ctx, stream, 1); launch_fill_blocks(lc, descs, ctx->infos.p, first, count, ctx->blocks[s].p, ctx->huf_items[s].p, ctx->fse_items[s].p, ctx->counters[s].p, ctx->totals_d.p + w, ctx->exec_order[s].p, exact_classes ? 1 : 0, resume); }
+        { ProfScope ps(ctx, stream, 1); launch_fill_blocks(lc, descs, ctx->infos.p, first, count, ctx->blocks[s].p, ctx->huf_items[s].p, ctx->fse_items[s].p, ctx->counters[s].p, ctx->totals_d.p + w, ctx->exec_order[s].p, resume); }
         if (!(flags & kFlagSizesOnly)) { ProfScope ps(ctx, stream, 2); launch_huff(lc, descs + first, ctx->blocks[s].p, ctx->huf_items[s].p, ctx->counters[s].p, (uint32_t)t.n_huf, ctx->lit[s].p, ctx->huf_recs[s].p, ctx->huf_cls0[s].p, ctx->huf_cls1[s].p, ctx->huf_big.p); }
         { ProfScope ps(ctx, stream, 3); launch_fse(lc, descs + first, ctx->blocks[s].p, ctx->fse_items[s].p, ctx->counters[s].p, (uint32_t)t.n_fse, ctx->seq[s].p); }
         if (overlap) {
@@ -759,6 +755,18 @@ extern "C" int czb_debug_guard_faults(czb_context* ctx, uint64_t* faults) {  // 
     unsigned long long v = 0;
     CZB_CUDA(ctx, cudaMemcpy(&v, ctx->guard_faults.p, sizeof v, cudaMemcpyDeviceToHost));
     *faults = v;
+    return CZS_OK;
+}
+static_assert(sizeof(czb_debug_wave_totals) == sizeof(WaveTotals) && offsetof(czb_debug_wave_totals, src_bytes) == offsetof(WaveTotals, src_bytes) &&
+              offsetof(czb_debug_wave_totals, frame_cls) == offsetof(WaveTotals, frame_cls) &&
+              offsetof(czb_debug_wave_totals, fse_cls) == offsetof(WaveTotals, fse_cls), "czb_debug_wave_totals mirrors WaveTotals");
+extern "C" int czb_debug_plan_waves(const czb_batch_plan* plan, uint64_t* wave_frames, uint64_t* n_waves, czb_debug_wave_totals* out,
+                                    uint64_t cap) {
+    if (!plan || (cap && !out)) return CZS_BAD_ARGUMENT;
+    if (wave_frames) *wave_frames = plan->W;
+    if (n_waves) *n_waves = plan->n_waves;
+    const uint64_t k = std::min<uint64_t>(cap, plan->totals.size());
+    if (k) memcpy(out, plan->totals.data(), k * sizeof(WaveTotals));
     return CZS_OK;
 }
 extern "C" int czb_debug_last_wave_counts(czb_context* ctx, uint64_t* n_blocks, uint64_t* lit_bytes, uint64_t* n_seq) {

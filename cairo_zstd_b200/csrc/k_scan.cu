@@ -117,30 +117,6 @@ __global__ void __launch_bounds__(128) k_scan_frames(const czb_frame_desc* __res
     }
 }
 
-// Recompute per-wave totals for a different wave size (planning retry; infos already scanned).
-__global__ void __launch_bounds__(128) k_wave_totals(const FrameInfo* __restrict__ infos, uint64_t n, uint64_t wave_frames,
-                                                      WaveTotals* __restrict__ totals) {
-    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    unsigned long long nb = 0, lb = 0, ns = 0, nh = 0, nf = 0;
-    if (i < n) { const FrameInfo& fi = infos[i]; nb = fi.n_blocks; lb = fi.lit_bytes; ns = fi.n_seq; nh = fi.n_huf; nf = fi.n_fse; }
-    nb = warp_sum_ull(nb); lb = warp_sum_ull(lb); ns = warp_sum_ull(ns); nh = warp_sum_ull(nh); nf = warp_sum_ull(nf);
-    if (lane_id() == 0 && i < n) {
-        WaveTotals* t = totals + i / wave_frames;
-        if (nb) atomicAdd(&t->n_blocks, nb);
-        if (lb) atomicAdd(&t->lit_bytes, lb);
-        if (ns) atomicAdd(&t->n_seq, ns);
-        if (nh) atomicAdd(&t->n_huf, nh);
-        if (nf) atomicAdd(&t->n_fse, nf);
-    }
-    // size classes for the new wave split (same per-frame classes as the scan)
-    if (i < n && infos[i].status == CZS_OK) {
-        const FrameInfo& fi = infos[i];
-        WaveTotals* t = totals + i / wave_frames;
-        atomicAdd(&t->frame_cls[fi.size_cls & 31u], 1u);
-        if (fi.n_fse) atomicAdd(&t->fse_cls[fi.fse_cls & 31u], fi.n_fse);
-    }
-}
-
 // Reserve n units in the per-class counter of class `cls` for this lane; lanes of a warp that share a class get
 // one atomic and consecutive ranges in lane order, so neighbouring frames stay neighbours in the work lists
 // (k_fse's 27 lanes then read neighbouring bitstreams: same DRAM pages, same TLB entries).
@@ -167,8 +143,7 @@ __global__ void __launch_bounds__(128) k_fill_blocks(const czb_frame_desc* __res
                                                       uint64_t first, uint64_t count, BlockDesc* __restrict__ blocks,
                                                       uint32_t* __restrict__ huf_items, uint32_t* __restrict__ fse_items,
                                                       WaveCounters* __restrict__ ctr, const WaveTotals* __restrict__ wt,
-                                                      uint32_t* __restrict__ exec_order, int exact_fse_classes,
-                                                      const FrameResume* __restrict__ resume) {
+                                                      uint32_t* __restrict__ exec_order, const FrameResume* __restrict__ resume) {
     // start of every size class in the work lists, largest class first
     __shared__ unsigned int frame_start[32], fse_start[32];
     if (threadIdx.x == 0) {
@@ -358,19 +333,12 @@ void launch_scan_frames(const LaunchCtx& lc, const czb_frame_desc* descs, FrameI
     k_scan_frames<<<(unsigned)((n + 127) / 128), 128, 0, lc.stream>>>(descs, infos, n, wave_frames, totals, resume);
     ++*lc.launches;
 }
-void launch_wave_totals(const LaunchCtx& lc, const FrameInfo* infos, uint64_t n, uint64_t wave_frames, WaveTotals* totals,
-                        uint64_t n_waves) {
-    if (!n) return;
-    cudaMemsetAsync(totals, 0, n_waves * sizeof(WaveTotals), lc.stream);
-    k_wave_totals<<<(unsigned)((n + 127) / 128), 128, 0, lc.stream>>>(infos, n, wave_frames, totals);
-    ++*lc.launches;
-}
 void launch_fill_blocks(const LaunchCtx& lc, const czb_frame_desc* descs, FrameInfo* infos, uint64_t first, uint64_t count,
                         BlockDesc* blocks, uint32_t* huf_items, uint32_t* fse_items, WaveCounters* counters,
-                        const WaveTotals* wave_totals, uint32_t* exec_order, int exact_fse_classes, const FrameResume* resume) {
+                        const WaveTotals* wave_totals, uint32_t* exec_order, const FrameResume* resume) {
     if (!count) return;
     k_fill_blocks<<<(unsigned)((count + 127) / 128), 128, 0, lc.stream>>>(descs, infos, first, count, blocks, huf_items, fse_items, counters,
-                                                                          wave_totals, exec_order, exact_fse_classes, resume);
+                                                                          wave_totals, exec_order, resume);
     ++*lc.launches;
 }
 void launch_header_results(const LaunchCtx& lc, const FrameInfo* infos, czb_frame_result* results, uint64_t n) {

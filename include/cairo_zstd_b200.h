@@ -275,6 +275,15 @@ int czb_debug_fd_device_work(const czb_frame_decoder* fd, uint64_t* runs, uint64
  * scratch, checked after every wave; returns how many guard bytes were found overwritten so far (0 = clean). */
 int czb_debug_guard_faults(czb_context* ctx, uint64_t* faults);
 int czb_debug_flow_watchdog(unsigned int* out16); /* -DCZB_FLOW_WATCHDOG builds: what a stuck wait loop of k_exec_flow recorded */
+/* The wave split a plan holds: frames per wave, number of waves, and per wave what the scan counted (blocks, bytes of Huffman
+ * literal scratch, sequence slots, Huffman and sequence sections, the compressed bytes the block walk covered in frames whose
+ * header parsed (the whole frame when it is valid), and the histograms of frames by compressed-size class and of sequence sections by sequence-count class, class = floor(log2)).
+ * Copies min(cap, n_waves) entries into out (out may be NULL when cap is 0). */
+typedef struct czb_debug_wave_totals {
+    uint64_t n_blocks, lit_bytes, n_seq, n_huf, n_fse, src_bytes;
+    uint32_t frame_cls[32], fse_cls[32];
+} czb_debug_wave_totals;
+int czb_debug_plan_waves(const czb_batch_plan* plan, uint64_t* wave_frames, uint64_t* n_waves, czb_debug_wave_totals* out, uint64_t cap);
 
 /* Number of kernel launches issued by this context since creation (bench bookkeeping). */
 uint64_t czb_kernel_launches(const czb_context* ctx);
