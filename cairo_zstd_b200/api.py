@@ -92,6 +92,7 @@ EXPORTS = [
     "czb_kernel_launches", "czb_profile_enable", "czb_profile_collect", "czs_status_name",
     "czb_split_frames_host", "czb_split_frames_device", "czb_frame_sizes_device", "czb_frame_sizes_host",
     "czb_dictionary_parse_host", "czb_plan_batch_device", "czb_plan_destroy", "czb_decode_batch_device_planned", "czb_debug_fd_device_work", "czb_debug_guard_faults", "czb_debug_flow_watchdog", "czb_debug_plan_waves", "czb_partition_frames", "czb_multi_create", "czb_multi_destroy", "czb_decode_batch_multi", "czb_multi_last_error",
+    "czb_verify_batch_device",
 ]
 
 _lib = None
@@ -114,6 +115,7 @@ def load_library():
     L.czb_last_error.argtypes = [vp]
     L.czb_last_error.restype = C.c_char_p
     L.czb_decode_batch_device.argtypes = [vp, vp, vp, u64, u32, vp]
+    L.czb_verify_batch_device.argtypes = [vp, vp, vp, u64, vp]
     L.czb_decode_batch_host.argtypes = [vp, P(FrameDesc), P(FrameResult), u64, u32]
     L.czb_decode_batch_host_packed.argtypes = [vp, vp, vp, vp, vp, vp, u64, u32]
     L.czb_frame_header_info_host.argtypes = [C.c_char_p, u64, P(FrameHeaderInfo)]
@@ -286,6 +288,11 @@ class Context:
     def decode_batch_device(self, descs_ptr: int, results_ptr: int, n: int, flags: int = 0, stream: int = 0):
         """descs_ptr/results_ptr: device addresses of czb_frame_desc[n] / czb_frame_result[n]."""
         self._check(self._L.czb_decode_batch_device(self._h, descs_ptr, results_ptr, n, flags, stream))
+
+    def verify_batch_device(self, descs_ptr: int, results_ptr: int, n: int, stream: int = 0):
+        """czb_verify_batch_device: decode into the context's scratch, XXH64 each output, keep only the results.
+        descs_ptr/results_ptr: device addresses of czb_frame_desc[n] / czb_frame_result[n]; dst / dst_cap are ignored."""
+        self._check(self._L.czb_verify_batch_device(self._h, descs_ptr, results_ptr, n, stream))
 
     def plan_batch_device(self, descs_ptr: int, n: int, stream: int = 0):
         """czb_plan_batch_device: returns an opaque plan handle (free with plan_destroy)."""

@@ -54,6 +54,13 @@ __global__ void k_check_guards(const uint8_t* a, const uint8_t* b, const uint8_t
     const uint8_t* p = t < 64 ? a : (t < 128 ? b : c);
     if (p && p[t & 63] != kGuardByte) atomicAdd(faults, 1ull);
 }
+// The output scratch of a verify call: its used end is known on the device only (k_place_outputs, ctl[0]).
+// faults == nullptr: write the 64 guard bytes there; else count those that changed.
+__global__ void k_out_guard(uint8_t* out, const unsigned long long* ctl, unsigned long long* faults) {
+    uint8_t* p = out + ctl[0] + threadIdx.x;
+    if (!faults) *p = kGuardByte;
+    else if (*p != kGuardByte) atomicAdd(faults, 1ull);
+}
 
 extern "C" int czb_abi_version(void) { return CZB_ABI_VERSION; }
 
@@ -128,10 +135,11 @@ extern "C" void czb_context_destroy(czb_context* ctx) {
     cudaSetDevice(ctx->device);
     cudaDeviceSynchronize();
     cudaFree(ctx->infos.p); cudaFree(ctx->totals_d.p); cudaFree(ctx->guard_faults.p); cudaFree(ctx->huf_big.p);
+    cudaFree(ctx->vdescs.p); cudaFree(ctx->out_sizes.p); cudaFree(ctx->out_cta.p);
     for (int s = 0; s < 2; s++) {
         cudaFree(ctx->exec_order[s].p); cudaFree(ctx->huf_cls0[s].p); cudaFree(ctx->huf_cls1[s].p); cudaFree(ctx->huf_recs[s].p);
         cudaFree(ctx->blocks[s].p); cudaFree(ctx->huf_items[s].p); cudaFree(ctx->fse_items[s].p); cudaFree(ctx->lit[s].p);
-        cudaFree(ctx->seq[s].p); cudaFree(ctx->counters[s].p);
+        cudaFree(ctx->seq[s].p); cudaFree(ctx->counters[s].p); cudaFree(ctx->out[s].p); cudaFree(ctx->out_ctl[s].p);
         if (ctx->ev_entropy[s]) cudaEventDestroy(ctx->ev_entropy[s]);
         if (ctx->ev_exec[s]) cudaEventDestroy(ctx->ev_exec[s]);
     }
@@ -190,11 +198,12 @@ extern "C" int czb_profile_collect(czb_context* ctx, double* ms, uint64_t* launc
     return CZS_OK;
 }
 
-static uint64_t wave_scratch_bytes(const WaveTotals& t) {
-    return t.n_blocks * sizeof(BlockDesc) + t.lit_bytes + t.n_seq * sizeof(Seq) + (t.n_huf + t.n_fse) * 4 + t.n_huf * (sizeof(HufRec) + 8);
+static uint64_t wave_scratch_bytes(const WaveTotals& t, bool verify) {
+    return entropy_scratch_bytes(t.n_blocks, t.lit_bytes, t.n_seq, t.n_huf, t.n_fse) + (verify ? verify_out_bytes(t.out_bound) : 0);
 }
 
 constexpr uint32_t kFlagSizesOnly = 0x80000000u;  // internal: scan + block walk + k_fse, then k_frame_sizes (czb_frame_sizes_*)
+constexpr uint32_t kFlagVerify = 0x40000000u;     // internal: outputs into the context's scratch, XXH64, no caller dst (czb_verify_batch_device)
 
 // The hot path.  descs/results are device arrays.  `resume` (device array, one entry per frame, or nullptr) is the handle's
 // way of continuing frames whose first blocks were executed by earlier calls (czb_handle.cu).
@@ -230,6 +239,14 @@ static int decode_batch_impl(czb_context* ctx, const czb_frame_desc* descs, czb_
     const bool capturing = cap_st != cudaStreamCaptureStatusNone;  // a captured call is ordered by the graph it becomes part of
     if (ctx->scratch_in_use && !capturing) CZB_CUDA(ctx, cudaStreamWaitEvent(stream, ctx->ev_scratch_free, 0));
     if (plan && plan->n != n) { ctx->last_error = "plan was made for a different batch"; return CZS_BAD_ARGUMENT; }
+    const bool verify = (flags & kFlagVerify) != 0;
+    if (verify) {  // every later stage reads the copy, whose dst / dst_cap k_place_outputs rewrites wave by wave
+        if ((rc = ensure(ctx, ctx->vdescs, n))) return rc;
+        CZB_CUDA(ctx, cudaMemcpyAsync(ctx->vdescs.p, descs, n * sizeof(czb_frame_desc), cudaMemcpyDeviceToDevice, stream));
+        descs = ctx->vdescs.p;
+    }
+    // verify: a frame whose scratch alone exceeds the budget gets CZS_UNSUPPORTED in the scan (DESIGN.md section 6)
+    const uint64_t frame_limit = verify ? ctx->budget / (ctx->no_overlap ? 1 : 2) : 0;
     if ((rc = ensure(ctx, ctx->infos, n))) return rc;
     if ((rc = ensure(ctx, ctx->totals_d, kMaxWaves))) return rc;
     if (!ctx->huf_big.p) {  // scratch for Huffman-weight FSE tables with an accuracy log above 9 (global memory, one warp at a time)
@@ -249,16 +266,17 @@ static int decode_batch_impl(czb_context* ctx, const czb_frame_desc* descs, czb_
     }
     // A retry (a wave's scratch over the budget) scans again with the smaller wave size: the scan is the only code that
     // produces wave totals, so a retried wave's totals are the ones a call starting at that wave size would see.
+    // Verify calls also count the output bound and may go below 128 frames per wave, down to one.
     while (!plan) {
         n_waves = (n + W - 1) / W;
         CZB_CUDA(ctx, cudaMemsetAsync(ctx->totals_d.p, 0, n_waves * sizeof(WaveTotals), stream));
-        { ProfScope ps(ctx, stream, 0); launch_scan_frames(lc, descs, ctx->infos.p, n, W, ctx->totals_d.p, resume); }
+        { ProfScope ps(ctx, stream, 0); launch_scan_frames(lc, descs, ctx->infos.p, n, W, ctx->totals_d.p, resume, verify, frame_limit); }
         launch_publish_totals(lc, ctx->totals_d.p, ctx->totals_h_dev, n_waves);
         CZB_CUDA(ctx, cudaStreamSynchronize(stream));
         uint64_t worst = 0;
-        for (uint64_t w = 0; w < n_waves; w++) worst = std::max(worst, wave_scratch_bytes(ctx->totals_h[w]));
-        if ((ctx->no_overlap ? 1 : 2) * worst <= ctx->budget || W <= 128 || (n + W / 2 - 1) / (W / 2) > kMaxWaves) break;
-        W = std::max<uint64_t>(128, (W / 2 + 127) / 128 * 128);
+        for (uint64_t w = 0; w < n_waves; w++) worst = std::max(worst, wave_scratch_bytes(ctx->totals_h[w], verify));
+        if ((ctx->no_overlap ? 1 : 2) * worst <= ctx->budget || W <= (verify ? 1u : 128u) || (n + W / 2 - 1) / (W / 2) > kMaxWaves) break;
+        W = W > 128 ? std::max<uint64_t>(128, (W / 2 + 127) / 128 * 128) : W / 2;
     }
     if (plan_out) {
         plan_out->n = n; plan_out->W = W; plan_out->n_waves = n_waves;
@@ -269,6 +287,7 @@ static int decode_batch_impl(czb_context* ctx, const czb_frame_desc* descs, czb_
         const WaveTotals& t = totals_host[w];
         mx.n_blocks = std::max(mx.n_blocks, t.n_blocks); mx.lit_bytes = std::max(mx.lit_bytes, t.lit_bytes);
         mx.n_seq = std::max(mx.n_seq, t.n_seq); mx.n_huf = std::max(mx.n_huf, t.n_huf); mx.n_fse = std::max(mx.n_fse, t.n_fse);
+        mx.out_bound = std::max(mx.out_bound, t.out_bound);
         if (t.n_blocks > 0xFFFFFF00ull) { ctx->last_error = "too many blocks in one wave"; return CZS_UNSUPPORTED; }
     }
     const int n_sets = (n_waves > 1 && !ctx->no_overlap) ? 2 : 1;
@@ -283,6 +302,14 @@ static int decode_batch_impl(czb_context* ctx, const czb_frame_desc* descs, czb_
         if ((rc = ensure(ctx, ctx->fse_items[s], mx.n_fse + 1))) return rc;
         if ((rc = ensure(ctx, ctx->lit[s], mx.lit_bytes + 64 + kGuardBytes))) return rc;
         if ((rc = ensure(ctx, ctx->seq[s], mx.n_seq + 2 + kGuardBytes / sizeof(Seq)))) return rc;
+        if (verify) {
+            if ((rc = ensure(ctx, ctx->out[s], verify_out_bytes(mx.out_bound) + kGuardBytes))) return rc;
+            if ((rc = ensure(ctx, ctx->out_ctl[s], 1))) return rc;
+        }
+    }
+    if (verify) {
+        if ((rc = ensure(ctx, ctx->out_sizes, W))) return rc;
+        if ((rc = ensure(ctx, ctx->out_cta, 2 * ((W + 127) / 128)))) return rc;
     }
 
     if (plan_out) return CZS_OK;  // scratch is sized, nothing else to do
@@ -337,16 +364,23 @@ static int decode_batch_impl(czb_context* ctx, const czb_frame_desc* descs, czb_
         { ProfScope ps(ctx, stream, 1); launch_fill_blocks(lc, descs, ctx->infos.p, first, count, ctx->blocks[s].p, ctx->huf_items[s].p, ctx->fse_items[s].p, ctx->counters[s].p, ctx->totals_d.p + w, ctx->exec_order[s].p, resume); }
         if (!(flags & kFlagSizesOnly)) { ProfScope ps(ctx, stream, 2); launch_huff(lc, descs + first, ctx->blocks[s].p, ctx->huf_items[s].p, ctx->counters[s].p, (uint32_t)t.n_huf, ctx->lit[s].p, ctx->huf_recs[s].p, ctx->huf_cls0[s].p, ctx->huf_cls1[s].p, ctx->huf_big.p); }
         { ProfScope ps(ctx, stream, 3); launch_fse(lc, descs + first, ctx->blocks[s].p, ctx->fse_items[s].p, ctx->counters[s].p, (uint32_t)t.n_fse, ctx->seq[s].p); }
+        if (verify) {  // exact slots in this set's output scratch (its own wave's bound, so the layout depends on the wave split only)
+            { ProfScope ps(ctx, stream, 7); launch_place_outputs(lc, ctx->infos.p, first, count, ctx->blocks[s].p, ctx->vdescs.p, results, ctx->out[s].p,
+                                                                  verify_out_bytes(t.out_bound), ctx->out_sizes.p, ctx->out_cta.p, ctx->out_ctl[s].p); }
+            if (ctx->guard) k_out_guard<<<1, kGuardBytes, 0, stream>>>(ctx->out[s].p, ctx->out_ctl[s].p, nullptr);
+        }
         if (overlap) {
             CZB_CUDA(ctx, cudaEventRecord(ctx->ev_entropy[s], stream));
             CZB_CUDA(ctx, cudaStreamWaitEvent(xs, ctx->ev_entropy[s], 0));
         }
         if (flags & kFlagSizesOnly) { ProfScope ps(ctx, xs, 7); launch_frame_sizes(lx, ctx->infos.p, first, count, ctx->blocks[s].p, results); }
         else { ProfScope ps(ctx, xs, 4); launch_exec(lx, ExecSide{ctx->big_stream, ctx->ev_big_fork, ctx->ev_big_join, use_flow, flow_wide, resume}, ctx->sm_count, descs, ctx->infos.p, first, count, n_big, n_exec, BigRule{(uint32_t)ctx->big_cls, (uint32_t)ctx->big_seq_bytes, (uint32_t)ctx->share_cls, share_bytes}, ctx->counters[s].p, ctx->exec_order[s].p, ctx->blocks[s].p, ctx->lit[s].p, ctx->seq[s].p, results); }
-        if ((flags & CZB_FLAG_VERIFY_CHECKSUM) && !(flags & kFlagSizesOnly)) { ProfScope ps(ctx, xs, 5); launch_xxh64(lx, descs, results, first, count); }
-        if (ctx->guard)
+        if ((flags & (CZB_FLAG_VERIFY_CHECKSUM | kFlagVerify)) && !(flags & kFlagSizesOnly)) { ProfScope ps(ctx, xs, 5); launch_xxh64(lx, descs, results, first, count); }
+        if (ctx->guard) {
             k_check_guards<<<1, 192, 0, xs>>>(ctx->lit[s].p + t.lit_bytes, reinterpret_cast<const uint8_t*>(ctx->seq[s].p + t.n_seq),
                                               reinterpret_cast<const uint8_t*>(ctx->blocks[s].p + t.n_blocks), ctx->guard_faults.p);
+            if (verify) k_out_guard<<<1, kGuardBytes, 0, xs>>>(ctx->out[s].p, ctx->out_ctl[s].p, ctx->guard_faults.p);
+        }
         if (overlap) CZB_CUDA(ctx, cudaEventRecord(ctx->ev_exec[s], xs));
         ctx->last_wave = t; ctx->last_wave_first = first; ctx->last_wave_count = count; ctx->last_set = s;
     }
@@ -365,6 +399,11 @@ static int decode_batch_impl(czb_context* ctx, const czb_frame_desc* descs, czb_
 extern "C" int czb_decode_batch_device(czb_context* ctx, const czb_frame_desc* descs, czb_frame_result* results, uint64_t n,
                                        uint32_t flags, void* stream_v) {
     return czb_decode_batch_device_resume(ctx, descs, results, n, flags & ~kFlagSizesOnly, stream_v, nullptr);
+}
+
+extern "C" int czb_verify_batch_device(czb_context* ctx, const czb_frame_desc* descs, czb_frame_result* results, uint64_t n,
+                                       void* stream_v) {
+    return decode_batch_impl(ctx, descs, results, n, kFlagVerify, stream_v, nullptr, nullptr, nullptr);
 }
 
 extern "C" int czb_plan_batch_device(czb_context* ctx, const czb_frame_desc* descs, uint64_t n, void* stream_v, czb_batch_plan** out) {
@@ -757,7 +796,7 @@ extern "C" int czb_debug_guard_faults(czb_context* ctx, uint64_t* faults) {  // 
     *faults = v;
     return CZS_OK;
 }
-static_assert(sizeof(czb_debug_wave_totals) == sizeof(WaveTotals) && offsetof(czb_debug_wave_totals, src_bytes) == offsetof(WaveTotals, src_bytes) &&
+static_assert(sizeof(czb_debug_wave_totals) == offsetof(WaveTotals, out_bound) && offsetof(czb_debug_wave_totals, src_bytes) == offsetof(WaveTotals, src_bytes) &&
               offsetof(czb_debug_wave_totals, frame_cls) == offsetof(WaveTotals, frame_cls) &&
               offsetof(czb_debug_wave_totals, fse_cls) == offsetof(WaveTotals, fse_cls), "czb_debug_wave_totals mirrors WaveTotals");
 extern "C" int czb_debug_plan_waves(const czb_batch_plan* plan, uint64_t* wave_frames, uint64_t* n_waves, czb_debug_wave_totals* out,
@@ -766,7 +805,7 @@ extern "C" int czb_debug_plan_waves(const czb_batch_plan* plan, uint64_t* wave_f
     if (wave_frames) *wave_frames = plan->W;
     if (n_waves) *n_waves = plan->n_waves;
     const uint64_t k = std::min<uint64_t>(cap, plan->totals.size());
-    if (k) memcpy(out, plan->totals.data(), k * sizeof(WaveTotals));
+    for (uint64_t w = 0; w < k; w++) memcpy(out + w, &plan->totals[w], sizeof(czb_debug_wave_totals));  // out_bound: verify calls only, never planned
     return CZS_OK;
 }
 extern "C" int czb_debug_last_wave_counts(czb_context* ctx, uint64_t* n_blocks, uint64_t* lit_bytes, uint64_t* n_seq) {

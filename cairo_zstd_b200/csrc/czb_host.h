@@ -37,6 +37,11 @@ struct czb_context {
     DevBuf<uint8_t> huf_big;    // FseBigScratch: Huffman-weight FSE tables with accuracy log 10..20
     DevBuf<uint8_t> lit[2];
     DevBuf<czb::Seq> seq[2];
+    // verify calls: the caller's descs with dst / dst_cap of the output scratch (k_place_outputs), the output scratch itself
+    // (double-buffered like the rest), and the placement's per-frame sizes, per-CTA sums and used end
+    DevBuf<czb_frame_desc> vdescs;
+    DevBuf<uint8_t> out[2];
+    DevBuf<unsigned long long> out_ctl[2], out_sizes, out_cta;
     cudaStream_t exec_stream = nullptr;
     cudaEvent_t ev_entropy[2] = {nullptr, nullptr}, ev_exec[2] = {nullptr, nullptr}, ev_fork = nullptr;
     cudaEvent_t ev_scratch_free = nullptr;  // recorded at the end of every batch call: the next call (any stream) waits on it

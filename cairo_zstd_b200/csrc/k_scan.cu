@@ -44,16 +44,19 @@ struct Walk {
 
 __device__ __forceinline__ uint64_t align16(uint64_t v) { return (v + 15) & ~15ull; }
 
+// VERIFY (verify calls): also the output bound, any wave size, and the per-frame scratch limit (launch_scan_frames).  The
+// decode instantiation is the kernel without them.
+template <bool VERIFY>
 __global__ void __launch_bounds__(128) k_scan_frames(const czb_frame_desc* __restrict__ descs, FrameInfo* __restrict__ infos,
                                                       uint64_t n, uint64_t wave_frames, WaveTotals* __restrict__ totals,
-                                                      const FrameResume* __restrict__ resume) {
+                                                      const FrameResume* __restrict__ resume, uint64_t frame_limit) {
     __shared__ unsigned int hist[2][32];
     if (threadIdx.x < 64) hist[threadIdx.x >> 5][threadIdx.x & 31] = 0;
     __syncthreads();
     const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     FrameInfo fi;
     memset(&fi, 0, sizeof fi);
-    uint64_t src_bytes = 0;
+    uint64_t src_bytes = 0, out_bound = 0;
     if (i < n) {
         const uint8_t* src = descs[i].src;
         uint64_t len = descs[i].src_len;
@@ -72,6 +75,7 @@ __global__ void __launch_bounds__(128) k_scan_frames(const czb_frame_desc* __res
                 parse_block_at(src, len, pos, pb);
                 fi.n_blocks++;
                 if (pb.hdr_status != CZS_OK) break;
+                if constexpr (VERIFY) out_bound += pb.type == BT_COMPRESSED ? (uint64_t)MAX_BLOCK_SIZE : (uint64_t)pb.size;
                 if (pb.type == BT_COMPRESSED && pb.pre_status == CZS_OK && fi.n_blocks > start_block) {
                     if (pb.lit_type >= LT_COMPRESSED) { fi.n_huf++; fi.lit_bytes += align16((uint64_t)pb.regen + 16); }
                     if (pb.seqhdr_status == CZS_OK && pb.n_seq) { fi.n_fse++; fi.n_seq += seq_slots(pb.n_seq); fi.n_seq_true += pb.n_seq; }
@@ -91,10 +95,41 @@ __global__ void __launch_bounds__(128) k_scan_frames(const czb_frame_desc* __res
             src_bytes = pos;
             fi.size_cls = size_class(pos);
             fi.fse_cls = fi.n_fse ? size_class(fi.n_seq_true / fi.n_fse) : 0u;
-            atomicAdd(&hist[0][fi.size_cls], 1u);
-            if (fi.n_fse) atomicAdd(&hist[1][fi.fse_cls], fi.n_fse);
+            if constexpr (VERIFY) {
+                out_bound = align16_u64(out_bound < MAX_FRAME_OUT ? out_bound : MAX_FRAME_OUT);
+                if (frame_limit && entropy_scratch_bytes(fi.n_blocks, fi.lit_bytes, fi.n_seq, fi.n_huf, fi.n_fse) + verify_out_bytes(out_bound) > frame_limit) {
+                    // too large for the budget even alone in a wave: reported like a header-level failure, nothing of it is planned
+                    const uint64_t fcs = fi.fcs, window = fi.window;
+                    memset(&fi, 0, sizeof fi);
+                    fi.status = CZS_UNSUPPORTED; fi.fcs = fcs; fi.window = window;
+                    src_bytes = 0; out_bound = 0;
+                }
+            }
+            if (fi.status == CZS_OK) {
+                if (!VERIFY || wave_frames % 128 == 0) {
+                    atomicAdd(&hist[0][fi.size_cls], 1u);
+                    if (fi.n_fse) atomicAdd(&hist[1][fi.fse_cls], fi.n_fse);
+                } else {  // a CTA may straddle waves
+                    WaveTotals* t = totals + i / wave_frames;
+                    atomicAdd(&t->frame_cls[fi.size_cls], 1u);
+                    if (fi.n_fse) atomicAdd(&t->fse_cls[fi.fse_cls], fi.n_fse);
+                }
+            }
         }
         infos[i] = fi;
+    }
+    if (VERIFY && wave_frames % 32 != 0) {  // a warp may straddle waves: every lane adds its own frame
+        if (i < n) {
+            WaveTotals* t = totals + i / wave_frames;
+            if (fi.n_blocks) atomicAdd(&t->n_blocks, (unsigned long long)fi.n_blocks);
+            if (fi.lit_bytes) atomicAdd(&t->lit_bytes, (unsigned long long)fi.lit_bytes);
+            if (fi.n_seq) atomicAdd(&t->n_seq, (unsigned long long)fi.n_seq);
+            if (fi.n_huf) atomicAdd(&t->n_huf, (unsigned long long)fi.n_huf);
+            if (fi.n_fse) atomicAdd(&t->n_fse, (unsigned long long)fi.n_fse);
+            if (src_bytes) atomicAdd(&t->src_bytes, (unsigned long long)src_bytes);
+            if (out_bound) atomicAdd(&t->out_bound, (unsigned long long)out_bound);
+        }
+        return;  // no __syncthreads below: the histograms went to global memory already
     }
     // per-wave totals: a warp never straddles waves (wave_frames is a multiple of 128)
     unsigned long long nb = warp_sum_ull(fi.n_blocks), lb = warp_sum_ull(fi.lit_bytes), ns = warp_sum_ull(fi.n_seq);
@@ -107,6 +142,11 @@ __global__ void __launch_bounds__(128) k_scan_frames(const czb_frame_desc* __res
         if (nh) atomicAdd(&t->n_huf, nh);
         if (nf) atomicAdd(&t->n_fse, nf);
         if (sb) atomicAdd(&t->src_bytes, sb);
+    }
+    if constexpr (VERIFY) {
+        const unsigned long long ob = warp_sum_ull(out_bound);
+        if (lane_id() == 0 && i < n && ob) atomicAdd(&totals[i / wave_frames].out_bound, ob);
+        if (wave_frames % 128 != 0) return;
     }
     // size-class histograms: one global atomic per class per CTA (a CTA never straddles waves)
     __syncthreads();
@@ -306,6 +346,146 @@ void launch_frame_sizes(const LaunchCtx& lc, const FrameInfo* infos, uint64_t fi
     ++*lc.launches;
 }
 
+// ---- output placement of verify calls (czb_verify_batch_device) ----------------------------------------------------------
+// After k_fse every frame's exact decoded size is known (the arithmetic of k_frame_sizes, up to the first block whose
+// literal or sequence stage failed: execution stops there).  k_out_sizes computes it per frame and sums each CTA's frames in
+// two classes; k_place_outputs gives every frame its slot by an exclusive scan and writes dst / dst_cap (= the exact size),
+// which the executors and k_xxh64 then read as they read a caller's descs.
+//   class 1: exact size <= the frame's bound (every block within MAX_BLOCK_SIZE): laid out first.  Their total is at most
+//            the wave's out_bound, so they always fit.
+//   class 2: more than the bound (a Compressed block that regenerates more than MAX_BLOCK_SIZE): laid out after class 1, as
+//            far as the scratch reaches; a frame beyond it gets CZS_UNSUPPORTED.
+// A frame whose exact size exceeds MAX_FRAME_OUT gets CZS_UNSUPPORTED with the fields the executors give it when dst_cap is
+// at least MAX_FRAME_OUT: blocks before the one that crosses the limit, bytes read up to there, nothing written.
+// sizes[t] = exact size | class << 32; cta_totals[2 b], [2 b + 1] = aligned bytes of class 1, 2 in CTA b.
+constexpr unsigned PLACE_THREADS = 128;
+
+__device__ __forceinline__ void unsupported_result(czb_frame_result* r, const FrameInfo& fi, uint32_t blocks_done, uint64_t bytes_read) {
+    czb_frame_result x;
+    memset(&x, 0, sizeof x);
+    x.status = CZS_UNSUPPORTED; x.blocks_decoded = blocks_done; x.bytes_read = bytes_read;
+    x.content_size = fi.fcs; x.window_size = fi.window; x.checksum_from_data = fi.checksum; x.has_checksum = fi.has_checksum;
+    *r = x;
+}
+
+// inclusive block-wide sums of two values (PLACE_THREADS threads); returns the CTA totals through tot_a / tot_b
+__device__ __forceinline__ void block_scan2(unsigned long long& a, unsigned long long& b, unsigned long long& tot_a, unsigned long long& tot_b) {
+    __shared__ unsigned long long wa[PLACE_THREADS / 32], wb[PLACE_THREADS / 32];
+    const unsigned lane = lane_id(), warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const unsigned long long x = __shfl_up_sync(0xFFFFFFFFu, a, o), y = __shfl_up_sync(0xFFFFFFFFu, b, o);
+        if ((int)lane >= o) { a += x; b += y; }
+    }
+    if (lane == 31) { wa[warp] = a; wb[warp] = b; }
+    __syncthreads();
+    unsigned long long pa = 0, pb = 0;
+    tot_a = 0; tot_b = 0;
+#pragma unroll
+    for (unsigned w = 0; w < PLACE_THREADS / 32; w++) {
+        if (w < warp) { pa += wa[w]; pb += wb[w]; }
+        tot_a += wa[w]; tot_b += wb[w];
+    }
+    a += pa; b += pb;
+    __syncthreads();
+}
+
+__global__ void __launch_bounds__(PLACE_THREADS) k_out_sizes(FrameInfo* __restrict__ infos, uint64_t first, uint64_t count,
+                                                             const BlockDesc* __restrict__ blocks, czb_frame_result* __restrict__ results,
+                                                             unsigned long long* __restrict__ sizes, unsigned long long* __restrict__ cta_totals) {
+    const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    unsigned long long a = 0, b = 0, packed = 0;
+    if (t < count) {
+        const FrameInfo fi = infos[first + t];
+        if (fi.status == CZS_OK) {
+            uint64_t out = 0, bound = 0, bytes_read = fi.hdr_len, read_at_cross = 0;
+            uint32_t cross = NONE32;
+            bool stopped = false;
+            for (uint32_t k = 0; k < fi.n_blocks; k++) {
+                const BlockDesc d = blocks[fi.block_base + k];
+                if (d.type == BT_RAW || d.type == BT_RLE) bound += d.size;  // the bound of k_scan_frames<true>, block for block
+                else if (d.type == BT_COMPRESSED) bound += MAX_BLOCK_SIZE;
+                if (stopped) continue;
+                uint64_t blk = 0, rd = 0;
+                if (d.type == BT_ERROR) { stopped = true; continue; }
+                if (d.type == BT_RAW) { blk = d.size; rd = 3ull + d.size; }
+                else if (d.type == BT_RLE) { blk = d.size; rd = 4; }
+                else {
+                    if (d.pre_status != CZS_OK || (d.lit_type >= LT_COMPRESSED && d.huf_status != CZS_OK) || d.seqhdr_status != CZS_OK ||
+                        (d.n_seq && d.fse_status != CZS_OK)) { stopped = true; continue; }
+                    blk = (uint64_t)d.regen + (d.n_seq ? d.ml_sum : 0u);
+                    rd = 3ull + d.size;
+                }
+                if (cross == NONE32 && out + blk > MAX_FRAME_OUT) { cross = k; read_at_cross = bytes_read; }
+                out += blk; bytes_read += rd;
+            }
+            bound = align16_u64(bound < MAX_FRAME_OUT ? bound : MAX_FRAME_OUT);
+            if (cross != NONE32) {
+                unsupported_result(results + first + t, fi, cross, read_at_cross);
+                infos[first + t].status = CZS_UNSUPPORTED;  // the executors and k_xxh64 skip it
+            } else {
+                const bool over = align16_u64(out) > bound;
+                (over ? b : a) = align16_u64(out);
+                packed = out | (over ? 2ull : 1ull) << 32;
+            }
+        }
+        sizes[t] = packed;
+    }
+    unsigned long long ta, tb;
+    block_scan2(a, b, ta, tb);
+    if (threadIdx.x == 0) { cta_totals[2 * blockIdx.x] = ta; cta_totals[2 * blockIdx.x + 1] = tb; }
+}
+
+__global__ void __launch_bounds__(PLACE_THREADS) k_place_outputs(FrameInfo* __restrict__ infos, uint64_t first, uint64_t count,
+                                                                 czb_frame_desc* __restrict__ descs, czb_frame_result* __restrict__ results,
+                                                                 uint8_t* __restrict__ out, uint64_t out_cap,
+                                                                 const unsigned long long* __restrict__ sizes,
+                                                                 const unsigned long long* __restrict__ cta_totals, unsigned long long* __restrict__ ctl) {
+    // bases of this CTA: class-1 bytes of the CTAs before it, the class-1 total, class-2 bytes of the CTAs before it
+    unsigned long long pre_a = 0, all_a = 0, pre_b = 0, all_b = 0;
+    for (unsigned j = threadIdx.x; j < gridDim.x; j += blockDim.x) {
+        const unsigned long long x = cta_totals[2 * j], y = cta_totals[2 * j + 1];
+        all_a += x; all_b += y;
+        if (j < blockIdx.x) { pre_a += x; pre_b += y; }
+    }
+    {
+        unsigned long long s0 = pre_a, s1 = pre_b, t0, t1;
+        block_scan2(s0, s1, t0, t1);
+        pre_a = t0; pre_b = t1;
+        s0 = all_a; s1 = all_b;
+        block_scan2(s0, s1, t0, t1);
+        all_a = t0; all_b = t1;
+    }
+    const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const unsigned long long packed = t < count ? sizes[t] : 0ull;
+    const uint32_t cls = (uint32_t)(packed >> 32);
+    const uint64_t exact = packed & 0xFFFFFFFFull;
+    unsigned long long a = cls == 1 ? align16_u64(exact) : 0ull, b = cls == 2 ? align16_u64(exact) : 0ull, ta, tb;
+    const unsigned long long own_a = a, own_b = b;
+    block_scan2(a, b, ta, tb);
+    if (blockIdx.x == 0 && threadIdx.x == 0) ctl[0] = all_a + all_b < out_cap ? all_a + all_b : out_cap;
+    if (!cls) return;
+    const uint64_t off = cls == 1 ? pre_a + a - own_a : all_a + pre_b + b - own_b;
+    if (off + exact > out_cap) {  // class 2 beyond the scratch
+        const FrameInfo fi = infos[first + t];
+        unsupported_result(results + first + t, fi, 0, fi.hdr_len);
+        infos[first + t].status = CZS_UNSUPPORTED;
+        return;
+    }
+    descs[first + t].dst = out + off;
+    descs[first + t].dst_cap = exact;
+}
+
+void launch_place_outputs(const LaunchCtx& lc, FrameInfo* infos, uint64_t first, uint64_t count, const BlockDesc* blocks,
+                          czb_frame_desc* descs, czb_frame_result* results, uint8_t* out, uint64_t out_cap,
+                          unsigned long long* sizes, unsigned long long* cta_totals, unsigned long long* ctl) {
+    if (!count) return;
+    const unsigned grid = (unsigned)((count + PLACE_THREADS - 1) / PLACE_THREADS);
+    k_out_sizes<<<grid, PLACE_THREADS, 0, lc.stream>>>(infos, first, count, blocks, results, sizes, cta_totals);
+    k_place_outputs<<<grid, PLACE_THREADS, 0, lc.stream>>>(infos, first, count, descs, results, out, out_cap, sizes, cta_totals, ctl);
+    *lc.launches += 2;
+}
+
 // Frame-boundary walk over a concatenated buffer, one thread (each frame starts where the previous one ends, so the walk
 // is one chain of dependent loads): skippable frames are stepped over (frame.cairo:160-166), every zstd frame's end is
 // found from its block headers (block_decoder.cairo:237-278) without decoding.  counts = {frames, skipped, consumed, status}.
@@ -328,9 +508,10 @@ void launch_publish_totals(const LaunchCtx& lc, const WaveTotals* totals_d, Wave
 }
 
 void launch_scan_frames(const LaunchCtx& lc, const czb_frame_desc* descs, FrameInfo* infos, uint64_t n, uint64_t wave_frames,
-                        WaveTotals* totals, const FrameResume* resume) {
+                        WaveTotals* totals, const FrameResume* resume, bool verify, uint64_t frame_limit) {
     if (!n) return;
-    k_scan_frames<<<(unsigned)((n + 127) / 128), 128, 0, lc.stream>>>(descs, infos, n, wave_frames, totals, resume);
+    if (verify) k_scan_frames<true><<<(unsigned)((n + 127) / 128), 128, 0, lc.stream>>>(descs, infos, n, wave_frames, totals, resume, frame_limit);
+    else k_scan_frames<false><<<(unsigned)((n + 127) / 128), 128, 0, lc.stream>>>(descs, infos, n, wave_frames, totals, resume, 0);
     ++*lc.launches;
 }
 void launch_fill_blocks(const LaunchCtx& lc, const czb_frame_desc* descs, FrameInfo* infos, uint64_t first, uint64_t count,

@@ -117,6 +117,24 @@ int czb_abi_version(void);
 int czb_decode_batch_device(czb_context* ctx, const czb_frame_desc* descs, czb_frame_result* results,
                             uint64_t n_frames, uint32_t flags, void* stream);
 
+/* Check frames without output buffers (`zstd -t`; the reference's _test_decode, src/tests/decoding.cairo:4-21, without
+ * collect()): decode every frame into scratch owned by the context, compute XXH64 low-32 of each output, and discard the
+ * output.  descs/results: DEVICE arrays as in czb_decode_batch_device; descs[i].dst and dst_cap are ignored and never
+ * written.  results[i] holds exactly what czb_decode_batch_device with CZB_FLAG_VERIFY_CHECKSUM and
+ * dst_cap = CZB_MAX_FRAME_OUTPUT would report (status, blocks_decoded, bytes_read, bytes_written = decoded size,
+ * content_size, window_size, checksum_from_data, checksum_calculated, has_checksum, finished).  Same stream and threading
+ * rules as that call.  Memory stays within the context's budget whatever the batch's decoded total: waves are sized by an
+ * upper bound on their output and may hold as few as one frame.  Differences, all CZS_UNSUPPORTED with the header's fields
+ * (content_size, window_size; the other fields 0 unless stated):
+ *   a. a frame whose output exceeds CZB_MAX_FRAME_OUTPUT, with the blocks_decoded / bytes_read the decode path reports for
+ *      it (even where that path would meet a malformed sequence before the limit);
+ *   b. a frame that alone, with its scratch and its output bound (MAX_BLOCK_SIZE = 128 KiB per Compressed block), exceeds
+ *      the budget (half the budget with CZB_OVERLAP=1);
+ *   c. a frame with a Compressed block that regenerates more than 128 KiB (the format's block maximum, which the reference
+ *      does not enforce), when its wave's output scratch cannot also hold it (bytes_read = its header length). */
+int czb_verify_batch_device(czb_context* ctx, const czb_frame_desc* descs, czb_frame_result* results,
+                            uint64_t n_frames, void* stream);
+
 /* The same without the planning read-back.  czb_plan_batch_device scans the frames once, synchronises `stream`, sizes the
  * context's scratch and keeps the wave split; czb_decode_batch_device_planned then decodes the SAME frames (same count, same
  * compressed bytes at the same or other addresses) without any host synchronisation: every kernel is only enqueued, so the
