@@ -9,6 +9,12 @@
 // per-block byte counts written by k_exec drive the incremental strategies (UptoBlocks / UptoBytes :202-214,
 // decode_from_to :245-326) and the window-limited draining (decode_buffer.cairo:135-203),
 // including RingBuffer::len ignoring `head` (ring_buffer.cairo:20-22).
+//
+// Failing calls follow the reference too: a decode_blocks call that fails consumes what read_block_header and
+// decompress_block slice off (3 bytes, 3 + Block_Size for a Compressed block whose body fails), and a block that fails in
+// sequence execution leaves the literals and matches before the failing check in the output.  Deviation: after an error
+// every later decode_blocks / decode_from_to returns the same status and changes nothing (the reference would read on with
+// half-updated scratch); read, collect and the getters keep working.
 #include <algorithm>
 #include <cstring>
 #include <vector>
@@ -58,6 +64,8 @@ struct czb_frame_decoder {
     uint64_t buf_len = 0;   // RingBuffer elements.len()
     uint64_t head = 0;      // RingBuffer.head
     uint64_t abs_base = 0;  // position in the frame's output of element 0 (moves on clear())
+    int32_t error = CZS_OK;          // first error of a decode call: later decode calls return it and change nothing
+    std::vector<uint8_t> partial;    // what the first failing block appends before its failing check (sequence execution)
 };
 
 #define FD_CUDA(fd, call)                                                                         \
@@ -86,6 +94,7 @@ static int fd_setup(czb_frame_decoder* fd, const uint8_t* src, uint64_t src_len,
     fd->uploaded = 0; fd->exec_blocks = 0; fd->hist[0] = 1; fd->hist[1] = 4; fd->hist[2] = 8; fd->exec_out = 0; fd->exec_bytes_read = fh.hdr_len;
     fd->frame_finished = false; fd->block_counter = 0; fd->bytes_read_counter = fh.hdr_len;
     fd->has_check_sum = false; fd->check_sum = 0; fd->buf_len = 0; fd->head = 0; fd->abs_base = 0;
+    fd->error = CZS_OK; fd->partial.clear();
     if (consumed) *consumed = fh.hdr_len;
     return CZS_OK;
 }
@@ -111,6 +120,64 @@ extern "C" void czb_fd_free(czb_frame_decoder* fd) {
     cudaSetDevice(fd->ctx->device);
     cudaFree(fd->d_src); cudaFree(fd->d_dst); cudaFree(fd->d_desc); cudaFree(fd->d_res); cudaFree(fd->d_resume);
     delete fd;
+}
+
+// Grow d_dst to at least `need` bytes, keeping the output of the executed blocks (later matches read it).
+static int fd_grow_dst(czb_frame_decoder* fd, uint64_t need, cudaStream_t st) {
+    if (need <= fd->d_dst_cap) return CZS_OK;
+    uint8_t* ndst = nullptr;
+    const uint64_t ncap = need + need / 2;
+    FD_CUDA(fd, cudaMalloc(reinterpret_cast<void**>(&ndst), ncap));
+    if (fd->d_dst && fd->exec_out) FD_CUDA(fd, cudaMemcpyAsync(ndst, fd->d_dst, fd->exec_out, cudaMemcpyDeviceToDevice, st));
+    FD_CUDA(fd, cudaStreamSynchronize(st));
+    cudaFree(fd->d_dst);
+    fd->d_dst = ndst; fd->d_dst_cap = ncap;
+    return CZS_OK;
+}
+
+static bool exec_stage_error(int32_t st) {
+    return st == CZS_EXEC_NOT_ENOUGH_BYTES_FOR_SEQUENCE || st == CZS_EXEC_ZERO_OFFSET || st == CZS_NOT_ENOUGH_BYTES_IN_DICTIONARY ||
+           st == CZS_OFFSET_TOO_BIG;
+}
+
+// execute_sequences (sequence_execution.cairo:12-83) on the host for block `b`, which failed in sequence execution, up to the
+// failing check: each sequence's literals, then its offset (the records hold it resolved, or symbolic on the history the block
+// started with), then the zero-offset and window checks, then its match.  The literals and records are copied back from the
+// context's scratch right after the run that produced them.
+static int fd_replay_failed_block(czb_frame_decoder* fd, const BlockDesc& b) {
+    czb_context* ctx = fd->ctx;
+    fd->partial.clear();
+    if (!b.n_seq) return CZS_OK;
+    std::vector<uint8_t> lits(b.regen);
+    if (b.lit_type == LT_RAW) {
+        if ((uint64_t)b.lit_src_off + b.regen > fd->acc.size()) return CZS_PANIC_INTERNAL;
+        memcpy(lits.data(), fd->acc.data() + b.lit_src_off, b.regen);
+    } else if (b.lit_type == LT_RLE) {
+        if (b.lit_src_off >= fd->acc.size()) return CZS_PANIC_INTERNAL;
+        memset(lits.data(), fd->acc[b.lit_src_off], b.regen);
+    } else if (b.regen) {
+        FD_CUDA(fd, cudaMemcpy(lits.data(), ctx->lit[ctx->last_set].p + b.lit_off, b.regen, cudaMemcpyDeviceToHost));
+    }
+    std::vector<Seq> seqs(b.n_seq);
+    FD_CUDA(fd, cudaMemcpy(seqs.data(), ctx->seq[ctx->last_set].p + b.seq_off, b.n_seq * sizeof(Seq), cudaMemcpyDeviceToHost));
+    const uint64_t base = fd->out_all.size();  // the output of the blocks before b
+    std::vector<uint8_t>& out = fd->partial;
+    uint64_t lp = 0;
+    for (const Seq r : seqs) {
+        const uint32_t ll = seq_ll(r), ml = seq_ml(r), f = seq_off29(r);
+        if (lp + ll > lits.size()) break;                                    // CZS_EXEC_NOT_ENOUGH_BYTES_FOR_SEQUENCE
+        out.insert(out.end(), lits.begin() + lp, lits.begin() + lp + ll);
+        lp += ll;
+        const uint64_t len = base + out.size();
+        if (f == OFF29_CLAMP) break;                                         // a far offset: beyond the output so far
+        const uint32_t o = off29_resolve(f, fd->hist[0], fd->hist[1], fd->hist[2]);
+        if (o == 0 || o > len) break;                                        // zero offset, offset beyond the output
+        for (uint32_t i = 0; i < ml; i++) {
+            const uint64_t at = base + out.size() - o;
+            out.push_back(at < base ? fd->out_all[at] : out[at - base]);
+        }
+    }
+    return CZS_OK;
 }
 
 // Decode the blocks of fd->acc that earlier runs have not executed yet and append to fd->blocks / fd->out_all.
@@ -150,15 +217,8 @@ static int fd_run_device(czb_frame_decoder* fd) {
     FD_CUDA(fd, cudaMemcpyAsync(fd->d_resume, &rs, sizeof rs, cudaMemcpyHostToDevice, st));
     czb_frame_result res{};
     for (;;) {
-        if (cap > fd->d_dst_cap) {  // grow, keeping the output of the executed blocks (later matches read it)
-            uint8_t* ndst = nullptr;
-            const uint64_t ncap = cap + cap / 2;
-            FD_CUDA(fd, cudaMalloc(reinterpret_cast<void**>(&ndst), ncap));
-            if (fd->d_dst && fd->exec_out) FD_CUDA(fd, cudaMemcpyAsync(ndst, fd->d_dst, fd->exec_out, cudaMemcpyDeviceToDevice, st));
-            FD_CUDA(fd, cudaStreamSynchronize(st));
-            cudaFree(fd->d_dst);
-            fd->d_dst = ndst; fd->d_dst_cap = ncap;
-        }
+        int grc = fd_grow_dst(fd, cap, st);
+        if (grc != CZS_OK) return grc;
         czb_frame_desc d{fd->d_src, n, fd->d_dst, fd->d_dst_cap};
         FD_CUDA(fd, cudaMemcpyAsync(fd->d_desc, &d, sizeof d, cudaMemcpyHostToDevice, st));
         int rc = czb_decode_batch_device_resume(ctx, fd->d_desc, fd->d_res, 1, 0, st, fd->d_resume);
@@ -176,6 +236,7 @@ static int fd_run_device(czb_frame_decoder* fd) {
     fd->blocks.resize(fd->exec_blocks);  // drop the record of a block that could not be read last time: it is re-examined
     uint64_t produced = fd->exec_out;
     bool complete = false;
+    const BlockDesc* failed = nullptr;
     for (uint64_t k = fd->exec_blocks; k < nb; k++) {
         const BlockDesc& b = bd[k];
         BlockRec r{};
@@ -194,7 +255,11 @@ static int fd_run_device(czb_frame_decoder* fd) {
             fd->hist[0] = b.hist_out[0]; fd->hist[1] = b.hist_out[1]; fd->hist[2] = b.hist_out[2];
             fd->exec_bytes_read += 3ull + r.body_bytes;
             fd->device_blocks++;
-        } else { r.status = res.status; fd->blocks.push_back(r); complete = true; break; }
+        } else {
+            r.status = res.status; fd->blocks.push_back(r); complete = true;
+            if (exec_stage_error(res.status)) failed = &b;
+            break;
+        }
         if (b.last) { complete = true; break; }
     }
     fd->run_complete = complete;
@@ -202,7 +267,8 @@ static int fd_run_device(czb_frame_decoder* fd) {
     fd->out_all.resize(produced);
     if (produced > fd->exec_out) FD_CUDA(fd, cudaMemcpy(fd->out_all.data() + fd->exec_out, fd->d_dst + fd->exec_out, produced - fd->exec_out, cudaMemcpyDeviceToHost));
     fd->exec_out = produced;
-    return CZS_OK;
+    fd->partial.clear();
+    return failed ? fd_replay_failed_block(fd, *failed) : CZS_OK;
 }
 
 static int fd_ensure_block(czb_frame_decoder* fd, uint32_t j) {
@@ -212,16 +278,43 @@ static int fd_ensure_block(czb_frame_decoder* fd, uint32_t j) {
     return fd_run_device(fd);
 }
 
-// One iteration of the block loop.  Returns CZS_OK and advances, or the block's error.
-static int fd_step_block(czb_frame_decoder* fd, bool* was_last) {
+// One iteration of the block loop.  Returns CZS_OK and advances, or the block's error.  *span_used = bytes of the caller's
+// span the iteration used, the reference's way: read_block_header moves 3 bytes on before it checks the header, and
+// decompress_block slices a Compressed block's content off before it parses it.  The header and the content are checked
+// against the current span first: a record of a block an earlier run executed beyond it is not used.
+static int fd_step_block(czb_frame_decoder* fd, bool* was_last, uint64_t* span_used) {
+    *span_used = 0;
+    const uint64_t pos = fd->bytes_read_counter;
+    if (fd->acc.size() - pos < 3) return CZS_PANIC_TRUNCATED;  // r.slice(0,3) (:240)
+    *span_used = 3;
+    ParsedBlock pb;
+    parse_block_at(fd->acc.data(), fd->acc.size(), pos, pb);
+    if (pb.hdr_status == CZS_PANIC_TRUNCATED) {  // the header is read and counted, the content is not there (:173, :98-146)
+        fd->bytes_read_counter += 3;
+        return CZS_PANIC_TRUNCATED;
+    }
+    if (pb.hdr_status != CZS_OK) return pb.hdr_status;  // FailedToReadBlockHeader: counters untouched (:166-171)
     int rc = fd_ensure_block(fd, fd->block_counter);
     if (rc != CZS_OK) return rc;
     if (fd->block_counter >= fd->blocks.size()) return CZS_PANIC_INTERNAL;
     const BlockRec& r = fd->blocks[fd->block_counter];
-    if (r.header_err) return r.status;     // FailedToReadBlockHeader: counters untouched (:166-171)
+    if (r.header_err) return r.status;
     fd->bytes_read_counter += 3;           // :173
-    if (r.status != CZS_OK) return r.status;  // FailedToReadBlockBody (:175-184)
+    if (r.status != CZS_OK) {              // FailedToReadBlockBody (:175-184)
+        if (pb.type == BT_COMPRESSED) *span_used += pb.content;
+        if (!fd->partial.empty()) {        // the literals and matches execute_sequences appended before its failing check
+            cudaStream_t st = fd->ctx->compute;
+            const uint64_t n = fd->partial.size();
+            if ((rc = fd_grow_dst(fd, fd->exec_out + n, st)) != CZS_OK) return rc;
+            FD_CUDA(fd, cudaMemcpy(fd->d_dst + fd->exec_out, fd->partial.data(), n, cudaMemcpyHostToDevice));  // hashed by get_calculated_checksum
+            fd->out_all.insert(fd->out_all.end(), fd->partial.begin(), fd->partial.end());
+            fd->buf_len += n;
+            fd->partial.clear();
+        }
+        return r.status;
+    }
     fd->bytes_read_counter += r.body_bytes;
+    *span_used += r.body_bytes;
     fd->buf_len += r.out_bytes;
     fd->block_counter++;
     *was_last = r.last;
@@ -238,16 +331,22 @@ static void fd_append_source(czb_frame_decoder* fd, const uint8_t* src, uint64_t
 extern "C" int czb_fd_decode_blocks(czb_frame_decoder* fd, const uint8_t* src, uint64_t src_len, uint64_t* consumed, int strategy,
                                     uint32_t n, int32_t* finished) {
     if (!fd || (!src && src_len)) return CZS_BAD_ARGUMENT;
-    const uint64_t start = fd->bytes_read_counter;
-    const uint64_t prev_acc = fd->acc.size();
+    if (fd->error != CZS_OK) {  // after an error: the same status, nothing consumed, nothing changed
+        if (consumed) *consumed = 0;
+        if (finished) *finished = fd->frame_finished ? 1 : 0;
+        return fd->error;
+    }
     fd_append_source(fd, src, src_len);
-    if (fd->acc.size() != prev_acc || fd->acc.size() != fd->decoded_acc_len) { /* new bytes: a later run may see more blocks */ }
+    uint64_t used = 0;
     const uint64_t size_before = fd->buf_len;
     const uint32_t blocks_before = fd->block_counter;
     int rc = CZS_OK;
     for (;;) {
         bool last = false;
-        if ((rc = fd_step_block(fd, &last)) != CZS_OK) break;
+        uint64_t step = 0;
+        rc = fd_step_block(fd, &last, &step);
+        used += step;
+        if (rc != CZS_OK) break;
         if (last) {
             fd->frame_finished = true;
             if (checksum_flag(fd)) {  // :189-199
@@ -257,14 +356,16 @@ extern "C" int czb_fd_decode_blocks(czb_frame_decoder* fd, const uint8_t* src, u
                 fd->check_sum = (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24);
                 fd->has_check_sum = true;
                 fd->bytes_read_counter += 4;
+                used += 4;
             }
             break;
         }
         if (strategy == CZB_STRATEGY_UPTO_BLOCKS) { if (fd->block_counter - blocks_before >= n) break; }
         else if (strategy == CZB_STRATEGY_UPTO_BYTES) { if (fd->buf_len - size_before >= n) break; }
     }
-    if (consumed) *consumed = fd->bytes_read_counter - start;
+    if (consumed) *consumed = used;
     if (finished) *finished = fd->frame_finished ? 1 : 0;
+    if (rc != CZS_OK) fd->error = rc;
     return rc;
 }
 
@@ -318,6 +419,7 @@ extern "C" int64_t czb_fd_read(czb_frame_decoder* fd, uint8_t* dst, uint64_t dst
 extern "C" int czb_fd_decode_from_to(czb_frame_decoder* fd, const uint8_t* src, uint64_t src_len, uint8_t* dst, uint64_t dst_cap,
                                      uint64_t* read_len, uint64_t* written) {
     if (!fd || !read_len || !written || (!src && src_len)) return CZS_BAD_ARGUMENT;
+    if (fd->error != CZS_OK) return fd->error;
     const uint64_t start = fd->bytes_read_counter;
     if (!is_finished(fd)) {
         fd_append_source(fd, src, src_len);
@@ -343,8 +445,9 @@ extern "C" int czb_fd_decode_from_to(czb_frame_decoder* fd, const uint8_t* src, 
             }
             (void)pb;
             bool last = false;
-            int rc = fd_step_block(fd, &last);
-            if (rc != CZS_OK) return rc;
+            uint64_t step = 0;
+            int rc = fd_step_block(fd, &last, &step);
+            if (rc != CZS_OK) { fd->error = rc; return rc; }
             if (last) {
                 fd->frame_finished = true;
                 if (checksum_flag(fd) && fd->acc.size() >= fd->bytes_read_counter + 4) {  // :307-316

@@ -254,7 +254,10 @@ int czb_fd_new(czb_context* ctx, const uint8_t* src, uint64_t src_len, uint64_t*
 int czb_fd_reset(czb_frame_decoder* fd, const uint8_t* src, uint64_t src_len, uint64_t* consumed);
 void czb_fd_free(czb_frame_decoder* fd);
 /* decode_blocks (:156-222).  src = the span right after what previous calls consumed.
- * *consumed = bytes used by this call; *finished = the Ok(bool). */
+ * *consumed = bytes used by this call, a failing call included (3 for a block-header error or a truncated
+ * body, 3 + Block_Size for a Compressed block whose body fails); *finished = the Ok(bool).
+ * After an error, every later decode_blocks / decode_from_to returns the same status and changes nothing
+ * (a deviation: the reference reads on with half-updated scratch); read, collect and the getters keep working. */
 int czb_fd_decode_blocks(czb_frame_decoder* fd, const uint8_t* src, uint64_t src_len, uint64_t* consumed,
                          int strategy, uint32_t n, int32_t* finished);
 /* collect (:224-231): returns 1 = Some (bytes in dst, *written set), 0 = None, <0 = -czs_status. */

@@ -1163,6 +1163,7 @@ int32_t oracle_fd_decode_from_to(oracle_fd* fd, const uint8_t* src, size_t src_l
     return 0;
 }
 void oracle_fd_getters(const oracle_fd* fd, oracle_result* res) { memset(res, 0, sizeof *res); fd_fill_result(fd, res); }
+void oracle_fd_buffer_state(const oracle_fd* fd, size_t* len, size_t* head) { *len = fd->scratch.buffer.len; *head = fd->scratch.buffer.head; }
 
 /* ------------------------------------------------------------------------- */
 /* Dictionary::decode_dict (src/decoding/dictionary.cairo:35-90): parsed, never applied by the reference  */

@@ -96,6 +96,8 @@ int32_t oracle_fd_decode_from_to(oracle_fd* fd, const uint8_t* src, size_t src_l
 /* read (:328-334) */
 size_t oracle_fd_read(oracle_fd* fd, uint8_t* dst, size_t dst_cap);
 void oracle_fd_getters(const oracle_fd* fd, oracle_result* res);
+/* the decode buffer's RingBuffer len and head: `read` reports an amount, len - head bounds what it drained */
+void oracle_fd_buffer_state(const oracle_fd* fd, size_t* len, size_t* head);
 
 /* ---- unit-level entry points used to pin the oracle against reference vectors ---- */
 uint64_t oracle_xxh64(const uint8_t* p, size_t len, uint64_t seed);

@@ -127,6 +127,7 @@ def lib():
                                                C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]
         L.oracle_fd_decode_from_to.restype = C.c_int32
         L.oracle_fd_getters.argtypes = [C.c_void_p, C.POINTER(OracleResult)]
+        L.oracle_fd_buffer_state.argtypes = [C.c_void_p, C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]
         _lib = L
     return _lib
 

@@ -526,9 +526,114 @@ def family_invalid(seed=9):
     return cases
 
 
+# ---------------------------------------------------------------------------
+# 9. resume points of the FrameDecoder handle
+# ---------------------------------------------------------------------------
+RESUME_OPTS = [dict(), dict(single_segment=False, window_log=10), dict(single_segment=False, window_log=10, checksum=False, fcs_width=0),
+               dict(checksum=False)]
+
+
+def family_resume(seed=10):
+    """Frames for the FrameDecoder handle fed block by block, where every device run starts after the blocks earlier runs
+    executed (FrameResume): a Raw / RLE prefix before each compressed block puts a resume point right in front of it.
+      - output before the resume point at every residue mod 16;
+      - the first sequence after it with offset 1 (a self-overlapping match starting on the resume point), 2..15, the first
+        byte of the frame (out0), out0 - 1 and the window;
+      - repeat codes first after it (ll = 0 and ll > 0, repeat 3 with ll = 0 = h0 - 1) on a history set before it;
+      - Repeat-mode tables whose FSE / RLE definition lies 1, 2 and 50 blocks back, over zero-output blocks (Raw(b""),
+        Rle(x, 0), a literals-only block of 0 bytes);
+    with window_log 10 (collect and read drain many windows) or single segment, with and without checksum and content size."""
+    rng = random.Random(seed)
+    cases = []
+
+    def gap(blocks, h, n):
+        blocks.append(Raw(_rb(rng, n)) if rng.random() < 0.5 else Rle(rng.randrange(256), n))
+        h.skip(n)
+
+    for r in range(16):
+        opts = RESUME_OPTS[r % 4]
+        window = 1 << 10 if "window_log" in opts else None
+        blocks, h = [], _Hist()
+        gap(blocks, h, 1024 + 16 * rng.randrange(8) + r)           # out0 = r (mod 16)
+        for k in range(4):
+            out0 = h.produced
+            o = [1 + (r + k) % 15, out0, out0 - 1, window or out0 - 2][k]
+            seqs = [h.add(0, o + 3 + rng.randrange(30) if k == 0 else 3 + rng.randrange(40), off(o))]
+            seqs += _rep_seqs(rng, h, 4 + rng.randrange(30))
+            tbl = ("predefined",) * 3 if k % 2 else (("fse", 6), ("fse", 5), ("fse", 6))
+            blocks.append(Seqs(lits_for(seqs, rng, rng.randrange(3)), seqs, tbl))
+            gap(blocks, h, 16 * rng.randrange(1, 40) + (r + 5 * k) % 16)
+        cases.append(case(f"resume-first-seq-r{r}", blocks, **opts))
+    # repeat codes first after the resume point, on a history the block before it set
+    for variant in range(4):
+        opts = RESUME_OPTS[variant]
+        blocks, h = [], _Hist()
+        gap(blocks, h, 700 + variant)
+        for ll0, v in REP_COMBOS:
+            setter = [h.add(2, 4, off(2 + rng.randrange(300))) for _ in range(3)]
+            blocks.append(Seqs(lits_for(setter, rng, 1), setter))
+            gap(blocks, h, 1 + rng.randrange(90))
+            ll = ll0 * (1 + rng.randrange(3))
+            if not h.ok(ll, v):
+                ll = 1
+            seqs = [h.add(ll, 3 + rng.randrange(20), v)] + _rep_seqs(rng, h, 3 + rng.randrange(10), only_rep=True)
+            blocks.append(Seqs(lits_for(seqs, rng, 0), seqs))
+            if variant % 2:
+                gap(blocks, h, rng.randrange(40))
+        cases.append(case(f"resume-rep-first-v{variant}", blocks, **opts))
+    # Repeat-mode tables defined 1, 2 and 50 blocks earlier, FSE and RLE definitions, zero-output blocks between
+    lls, mls, offs = (1, 2, 5, 9), (3, 4, 7, 10), range(5, 29)     # offsets 5..28: offset codes 3 and 4
+
+    def table_block(h, rle):
+        if rle:
+            seqs = [h.add(5, 7, off(rng.choice(offs))) for _ in range(12)]
+            return Seqs(lits_for(seqs, rng, 2), seqs, (("rle", S.ll_code(5)), ("fse", 5), ("rle", S.ml_code(7))))
+        seqs = [h.add(a, b, off(o)) for a in lls for b in mls for o in (6, 20)]
+        rng.shuffle(seqs)
+        return Seqs(lits_for(seqs, rng, 1), seqs, (("fse", 6), ("fse", 5), ("fse", 6)))
+
+    for n_between in (1, 2, 50):
+        for rle in (False, True):
+            opts = RESUME_OPTS[(n_between + rle) % 4]
+            blocks, h = [], _Hist()
+            gap(blocks, h, 512 + n_between)
+            for _ in range(2):
+                blocks.append(table_block(h, rle))
+                for j in range(n_between):
+                    z = j % 4
+                    if z == 0:
+                        blocks.append(Raw(b""))
+                    elif z == 1:
+                        blocks.append(Rle(0x5C, 0))
+                    elif z == 2:
+                        blocks.append(Seqs(b"", []))
+                    else:
+                        gap(blocks, h, 1 + rng.randrange(60))
+                if rle:
+                    seqs = [h.add(5, 7, off(rng.choice(offs))) for _ in range(9)]
+                else:
+                    seqs = [h.add(rng.choice(lls), rng.choice(mls), off(rng.choice((6, 20)))) for _ in range(20)]
+                blocks.append(Seqs(lits_for(seqs, rng, 3), seqs, ("repeat", "repeat", "repeat")))
+                blocks.append(Seqs(b"", []))
+            cases.append(case(f"resume-repeat-tables-{n_between}-{'rle' if rle else 'fse'}", blocks, **opts))
+    # no content size, and a late block that regenerates more than 128 KiB: the handle's output bound for the blocks it has
+    # not run is too small in the middle of the frame; the next block matches into output written before that
+    h = _Hist()
+    blocks = [Raw(_rb(rng, 3000)), Rle(0x21, 5000)]
+    h.skip(8000)
+    s = [h.add(0, 1000 + rng.randrange(40), off(1 + rng.randrange(7000))) for _ in range(140)]
+    blocks += [Seqs(b"", s), Raw(_rb(rng, 100))]
+    h.skip(100)
+    s = [h.add(1, 200, off(h.produced + 1 - rng.randrange(1, 2000))) for _ in range(5)]
+    blocks.append(Seqs(lits_for(s, rng, 2), s))
+    cases.append(case("resume-late-block-over-128k", blocks, libzstd=None, single_segment=False, window_log=20, fcs_width=0))
+    return cases
+
+
 FAMILIES = {
     "chunks": family_chunks, "reach": family_reach, "repeat": family_repeat, "big": family_big, "flow": family_flow,
     "batch": family_batch, "tables": lambda: family_tables() + risky_pair(), "invalid": family_invalid,
+    "resume": family_resume,
 }
 
 _cache = {}

@@ -2,13 +2,21 @@
 FrameDecoderStateTrait::reset incl. the 100 MiB WindowSizeTooBig check (src/frame_decoder.cairo:78-105, :92-94),
 FrameDecoderTrait::read (:328-334) and decode_from_to (:245-326) with small feeds, including the
 RingBuffer::len quirk (src/decoding/ring_buffer.cairo:20-22), call by call against the oracle's restatement
-of the same state machine (oracle_fd_*).  Everything goes through the C ABI (czb_fd_*)."""
+of the same state machine (oracle_fd_*).  Everything goes through the C ABI (czb_fd_*).
+
+The tests after those run tests/fdscript.py's scripts on the handle and the oracle call by call: every device run of the
+handle RESUMES after the blocks earlier runs executed (FrameResume), under each executor: k_exec ("default", "warp": every
+frame on the per-warp path), k_exec_flow narrow and wide, k_exec_big.  Every case of every seqfamilies / huffamilies family
+block by block (the seams scripts), ragged / chunked / shrink / reset scripts over samples of them, corpus frames and libzstd
+frames, and the handle's behaviour on failing calls."""
 import ctypes as C
 import struct
 
 import pytest
 
+import fdscript as D
 import oracle_lib as O
+import seqfamilies as F
 import cairo_zstd_b200 as czb
 from cairo_zstd_b200.frame_decoder import ByteSlice
 from gpu_common import sha
@@ -199,3 +207,154 @@ def test_read_after_partial_decode_follows_the_ring_buffer_len_quirk(corpus):
             break
     assert dec.is_finished()
     L.oracle_fd_free(ofd)
+
+
+# ---------------------------------------------------------------------------
+# scripts, side by side with the oracle, under every executor
+# ---------------------------------------------------------------------------
+MODES = ["default", "warp", "flow-narrow", "flow-wide", "big"]
+
+
+def _env(monkeypatch, mode, **knobs):
+    """A context whose executor choice is forced (as test_gpu_verify.py's _env)."""
+    if mode == "warp":
+        monkeypatch.setenv("CZB_BIG_CLS", "31"); monkeypatch.setenv("CZB_SHARE_CLS", "31")
+    elif mode != "default":
+        monkeypatch.setenv("CZB_BIG_CLS", "0"); monkeypatch.setenv("CZB_BIG_SEQ_BYTES", "0")
+    if mode == "flow-wide":
+        monkeypatch.setenv("CZB_FLOW_WIDE", "1")
+    if mode == "big":
+        monkeypatch.setenv("CZB_BIG_FLOW", "0")
+    for k, v in knobs.items():
+        monkeypatch.setenv(k, str(v))
+    return czb.Context(0)
+
+
+def _watchdog_clear():
+    wd = (C.c_uint32 * 16)()
+    czb.load_library().czb_debug_flow_watchdog(wd)
+    assert wd[0] == 0, list(wd)
+
+
+def _seams(ctx, c, label):
+    lay = D.layout(c.frame)
+    res = D.run(c.frame, D.seams(lay), ctx, label=f"{c.name}/{label}")
+    D.check(c, "seams", res.epochs[0])
+    if not lay.failing:   # one device run per block, and every block executed once
+        assert res.device_work == (len(lay.blocks), len(lay.blocks)), (c.name, res.device_work, len(lay.blocks))
+    return res
+
+
+@pytest.mark.parametrize("mode", MODES)
+@pytest.mark.parametrize("kind,name", D.family_names())
+def test_seams_every_family_case(monkeypatch, kind, name, mode):
+    """Every case, valid and invalid, decode_blocks(UptoBlocks(1)) per block with the span ending on that block's end: each
+    device run executes one block on the output, history and counters of the runs before it."""
+    ctx = _env(monkeypatch, mode)
+    for c in D.family_cases(kind, name):
+        _seams(ctx, c, mode)
+    if mode != "default":
+        _watchdog_clear()
+    ctx.close()
+
+
+def _script_frames(corpus):
+    """(case, seed) of the ragged / chunked / shrink scripts: a fixed sample of each family, corpus frames, libzstd frames."""
+    out = []
+    for kind, name in D.family_names():
+        out += [(c, k) for k, c in enumerate(D.sample(D.family_cases(kind, name)))]
+    for name in D.CORPUS:
+        i = _idx(corpus, name)
+        f = corpus.frame(i)
+        out.append((F.Case(name, f, O.decode_frame(f, dst_cap=corpus.index[i]["orig_len"] + 64)[1], 0), i))
+    for wl, (f, data) in D.libzstd_frames().items():
+        out.append((F.Case(f"libzstd-wl{wl}", f, data, len(data)), wl))
+    return out
+
+
+@pytest.mark.parametrize("mode", ["default", "warp"])
+def test_ragged_chunked_shrink_scripts(monkeypatch, corpus, mode):
+    """Span ends inside headers, bodies and the trailer under every strategy form; decode_from_to in chunks of 1, 3, 7, 4096
+    bytes and a mix; spans that end before blocks the device already ran (the call fails as the oracle's does).  Under the
+    two k_exec forms only (about 40 s each); the seams scripts cover every executor."""
+    ctx = _env(monkeypatch, mode)
+    for c, seed in _script_frames(corpus):
+        lay = D.layout(c.frame)
+        for sname, script in D.scripts(lay, seed):
+            if sname == "chunked1" and len(c.frame) > 40000:
+                continue
+            res = D.run(c.frame, script, ctx, label=f"{c.name}/{sname}/{mode}")
+            D.check(c, sname, res.epochs[0])
+    if mode != "default":
+        _watchdog_clear()
+    ctx.close()
+
+
+@pytest.mark.parametrize("mode", ["default", "big"])
+def test_reset_in_the_middle_of_a_frame(monkeypatch, corpus, mode):
+    """reset after a device run that executed blocks beyond block_counter, the other frame, then the first again block by
+    block."""
+    ctx = _env(monkeypatch, mode)
+    pairs = [(F.cases("resume")[0], F.cases("repeat")[3]), (F.cases("resume")[-1], F.cases("resume")[17])]
+    z = corpus.frame(_idx(corpus, "z000033"))
+    pairs.append((F.cases("reach")[5], F.Case("z000033", z, O.decode_frame(z, dst_cap=1 << 24)[1], 0)))
+    for a, b in pairs:
+        res = D.run([a.frame, b.frame], D.reset(D.layout(a.frame)), ctx, label=f"reset {a.name} {b.name}")
+        assert [e.frame for e in res.epochs] == [0, 1, 0]
+        assert bytes(res.epochs[1].drained) == D.expected_output(b) and bytes(res.epochs[2].drained) == a.expected
+    ctx.close()
+
+
+@pytest.mark.parametrize("knob", ["CZB_OVERLAP", "CZB_GUARD"])
+def test_resume_scripts_with_overlap_and_guard(monkeypatch, corpus, knob):
+    ctx = _env(monkeypatch, "default", **{knob: 1})
+    for c in F.cases("resume"):
+        _seams(ctx, c, knob)
+    f = corpus.frame(_idx(corpus, "z000033"))
+    res = D.run(f, D.ragged(D.layout(f), __import__("random").Random(5)), ctx, label=f"z000033/ragged/{knob}")
+    assert res.epochs[0].finished
+    if knob == "CZB_GUARD":
+        assert ctx.guard_faults() == 0
+    ctx.close()
+
+
+def test_failing_calls_consume_what_the_oracle_consumes():
+    """A header error or a truncated body moves the caller's span 3 bytes on, a Compressed block whose body fails 3 +
+    Block_Size; bytes_read_from_source counts 3 for a failing body, nothing for a header error.  Both call forms."""
+    ctx = czb.Context(0)
+    for frame, _, status, _, _ in D.failing_frames():
+        for script in ([("blocks", None, D.ALL, 0), ("read",), ("collect",), ("blocks", None, D.ALL, 0), ("fromto", 64)],
+                       [("blocks", None, D.UPTO_BLOCKS, 1), ("blocks", None, D.UPTO_BYTES, 1), ("read",)],
+                       [("fromto*", [1, 5, 4096])]):
+            res = D.run(frame, script, ctx, label=status)
+            if script[0][0] != "fromto*" or status != "CZS_PANIC_TRUNCATED":   # decode_from_to waits for a truncated body
+                assert czb.status_name(res.epochs[0].status) == status, (status, script[0])
+    ctx.close()
+
+
+def test_block_failing_in_execution_leaves_its_partial_output():
+    """execute_sequences appends each sequence's literals before its offset checks, and the matches before the failing one:
+    after the offset check fails the 300-byte Raw block is followed by 3 literals, a 4-byte match and 2 more literals
+    (309 bytes), in collect(), read() and get_calculated_checksum alike."""
+    ctx = czb.Context(0)
+    c = next(c for c in F.cases("invalid") if c.name == "invalid-offset-past-start")
+    for script in ([("fromto*", [4096]), ("collect",)], D.seams(D.layout(c.frame)),
+                   [("blocks", None, D.ALL, 0), ("read",), ("read",), ("collect",)]):
+        ep = D.run(c.frame, script, ctx, label=c.name).epochs[0]
+        assert czb.status_name(ep.status) == c.expected == "CZS_OFFSET_TOO_BIG"
+        assert len(ep.drained) == 309
+    ctx.close()
+
+
+def test_decode_calls_after_an_error_change_nothing():
+    """After a failing call every later decode_blocks / decode_from_to returns the same status, consumes nothing and changes
+    no getter, whatever span it is given; read, collect and the getters keep working (DESIGN.md section 6)."""
+    ctx = czb.Context(0)
+    for c in F.cases("invalid"):
+        if D.expected_output(c) is not None:
+            continue
+        script = [("fromto", 1 << 20), ("blocks", None, D.ALL, 0), ("blocks", None, D.UPTO_BLOCKS, 1), ("fromto", 1 << 20),
+                  ("read",), ("can_collect",), ("blocks", 0, D.ALL, 0), ("collect",), ("fromto", 3), ("read",)]
+        ep = D.run(c.frame, script, ctx, label=c.name).epochs[0]
+        assert czb.status_name(ep.status) == c.expected
+    ctx.close()
