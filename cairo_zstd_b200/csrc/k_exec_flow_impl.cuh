@@ -407,9 +407,11 @@ __global__ void __launch_bounds__(FLOW_WARPS * 32, FLOW_P_MIN_CTAS) k_exec_flow(
                     uint32_t idle_spins = 0;
                     for (uint32_t round = 0; __any_sync(0xFFFFFFFFu, pending); round++) {
                         uint32_t r_now = 0, ab = 0;
-                        if (lane == 0) { r_now = vld(&sm.retired_out); ab = vld(&sm.abort); }
+                        if (lane == 0) { r_now = vld(&sm.retired_out); ab = vld(&sm.abort) | (vld(&sm.err_chunk) < c ? 1u : 0u); }
                         r_now = __shfl_sync(0xFFFFFFFFu, r_now, 0);
-                        if (__shfl_sync(0xFFFFFFFFu, ab, 0)) break;  // somebody gave up: the frame fails, nothing here matters any more
+                        // somebody gave up, or an earlier chunk failed -- it writes nothing, so a source that reaches into its span never
+                        // gets its ready bits: the frame fails with that chunk's status, nothing here matters any more
+                        if (__shfl_sync(0xFFFFFFFFu, ab, 0)) break;
                         bool ready = false;
                         if (pending) {
                             if (s_end <= lo_abs || s_end <= r_now) ready = true;

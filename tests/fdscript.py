@@ -519,14 +519,21 @@ def scripts(lay, seed, other=None):
 # frames, and what the caller must get from them
 # ---------------------------------------------------------------------------
 def family_names():
+    import fsefamilies as X
     import huffamilies as HF
     import seqfamilies as F
-    return [("seq", n) for n in sorted(F.FAMILIES)] + [("huf", n) for n in sorted(HF.FAMILIES)]
+    return [("seq", n) for n in sorted(F.FAMILIES)] + [("huf", n) for n in sorted(HF.FAMILIES)] + [("fse", n) for n in sorted(X.FAMILIES)]
+
+
+FSE_SAMPLED = ("desc", "counts")    # thousands of blocks (a table covered over up to 512 Repeat blocks): a fixed sample
 
 
 def family_cases(kind, name):
+    import fsefamilies as X
     import huffamilies as HF
     import seqfamilies as F
+    if kind == "fse":
+        return sample(X.cases(name), 16) if name in FSE_SAMPLED else X.cases(name)
     return (F if kind == "seq" else HF).cases(name)
 
 

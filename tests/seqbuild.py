@@ -145,9 +145,8 @@ def reference_decode(blocks, window=None):
                 start = len(out) - o
                 if o >= ml:
                     out += out[start:start + ml]
-                else:
-                    for k in range(ml):  # self-overlap: byte by byte
-                        out.append(out[start + k])
+                else:  # self-overlap: the match repeats the o bytes it starts on
+                    out += (out[start:] * (ml // o + 1))[:ml]
             out += lits[pos:]
     return bytes(out)
 

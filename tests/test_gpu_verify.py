@@ -7,6 +7,7 @@ import ctypes as C
 import numpy as np
 import pytest
 
+import fsefamilies as XF
 import huffamilies as HF
 import largeframes as LF
 import seqfamilies as SF
@@ -126,7 +127,7 @@ def _configs():
 
 def _families():
     frames, caps = [], []
-    for mod in (SF, HF):
+    for mod in (SF, HF, XF):
         for name in mod.FAMILIES:
             for c in mod.cases(name):
                 frames.append(c.frame)

@@ -18,6 +18,7 @@ import numpy as np
 import pytest
 
 import handmade as H
+import fsefamilies as X
 import huffamilies as HF
 import oracle_lib as O
 import seqbuild as S
@@ -275,7 +276,7 @@ def large_frames():
 def build_pool(corpus):
     p = Pool()
     p.add("corpus", [corpus.frame(i) for i in range(len(corpus))], [e["orig_len"] for e in corpus.index])
-    for fam, mod in ((F, "seq"), (HF, "huf")):
+    for fam, mod in ((F, "seq"), (HF, "huf"), (X, "seq")):
         for name in sorted(fam.FAMILIES):
             for c in fam.cases(name):
                 p.add(mod if isinstance(c.expected, bytes) else mod + "-bad", [c.frame], [c.cap])
